@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- headline benchmark of the B200-native interior-point path.
 
-    python bench.py --gpus N --steps K --warmup W [--workload C1|C2|C3] [--impl reference]
+    python bench.py --gpus N --steps K --warmup W [--workload C1|C2|C3] [--impl reference] [--dump-outputs DIR]
 
 A "step" is ONE COMPLETE SOLVE (blind start -> Optimal) of the workload LP, i.e. one pass of the
 hot path (`InteriorPoint::solve`, /root/reference/src/solvers/interior_point/mod.rs:161-240) over
@@ -27,6 +27,11 @@ one bounded sample of iterations in the reference arm (`details.step`).
 
 N > 1: strong scaling -- the same LP with A column-sharded over the ranks (SURVEY.md 8e), NCCL
 all-reduce of M and of the A.w products.
+
+`--dump-outputs DIR` writes, after the timed steps, what the last timed step returned to its caller as
+DIR/<name>.npy in float64: `x`, `fun` and `iteration` of the solve (C4: `x`, `fun`, `iteration` and `status` of
+every LP, rows in batch order, with `lp_index`).  The inputs are seeded, so two builds run with the same arguments
+can be compared output for output.
 """
 from __future__ import annotations
 
@@ -290,6 +295,35 @@ def _sync_max_ms(torch, dist, ms):
     return float(t.item())
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, arrays):
+    """--dump-outputs: each array as <out_dir>/<name>.npy in float64 (64 MB at most in all)."""
+    arrays = {k: np.asarray(v, dtype=np.float64) for k, v in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise ValueError("--dump-outputs: %d bytes exceed the limit of %d" % (total, DUMP_LIMIT_BYTES))
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+
+
+def dump_solve(out_dir, res):
+    dump_outputs(out_dir, {"x": res.x(), "fun": res.fun(), "iteration": res.iteration()})
+
+
+def _gather_rows(torch, dist, t, per, total):
+    """Rows of a batch sharded over the ranks in blocks of `per`, on the host in batch order (every rank calls)."""
+    if dist is None:
+        return t.cpu().numpy()
+    pad = torch.zeros((per,) + tuple(t.shape[1:]), dtype=t.dtype, device=t.device)
+    pad[: t.shape[0]] = t
+    parts = [torch.empty_like(pad) for _ in range(dist.get_world_size())]
+    dist.all_gather(parts, pad)
+    return torch.cat(parts)[:total].cpu().numpy()
+
+
 def _roofline(prof_sum, m, n_loc, peak_measured=None):
     """K1 roofline.  `achieved` counts the flop the kernel EXECUTES: m(m+1) * syrk_cols, where syrk_cols
     is n minus the trailing slack columns that liblpb200 folds into the diagonal of M instead of
@@ -426,6 +460,8 @@ def run_device_synthetic(args, torch, dist, rank, local_rank, world, stream, m, 
     torch.cuda.synchronize()
     gen_s = time.perf_counter() - t0
     ms, total_iters, launches, prof_sum, clocks, res = _timed_solves(args, torch, dist, solver, rp, local_rank)
+    if args.dump_outputs and rank == 0:
+        dump_solve(args.dump_outputs, res)
     value = total_iters / (ms * 1e-3)
     peak_holder = [measure_peak(rp) if rank == 0 else None]
     rp.close()
@@ -529,6 +565,14 @@ def run_batched(args, torch, dist, rank, local_rank, world, stream):
         dist.all_reduce(n_ok)
     total_iters = float(its.item())
     value = total_iters * args.steps / (ms * 1e-3)
+    if args.dump_outputs:
+        outs = [_gather_rows(torch, dist, t, per, batch) for t in (dx, dfun, dit, dst)]
+        if rank == 0:
+            rows = np.arange(batch)
+            if batch * (n + 4) * 8 > DUMP_LIMIT_BYTES:  # a fixed, seeded sample of the LPs
+                rows = np.sort(np.random.default_rng(0).choice(batch, DUMP_LIMIT_BYTES // ((n + 4) * 8), replace=False))
+            dump_outputs(args.dump_outputs, dict(zip(("lp_index", "x", "fun", "iteration", "status"),
+                                                     [rows] + [o[rows] for o in outs])))
     # e2e: host arrays in, host arrays out through lp_b200.solve_batched (H2D of A, b, c + D2H of x, fun, ...)
     barrier()
     t0 = time.perf_counter()
@@ -606,7 +650,13 @@ def main():
     ap.add_argument("--potrf-dist", type=int, default=2, choices=[0, 1, 2],
                     help="N > 1: 2 = distributed Cholesky, two broadcasts per panel + side-stream potf2 (default), "
                          "1 = one broadcast per panel, 0 = replicated on every rank")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step returned as DIR/<name>.npy (float64)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs writes the outputs of the product arm (--impl b200)")
     m, n = WORKLOADS[args.workload]
 
     if args.impl == "reference":
@@ -696,6 +746,8 @@ def main():
         t = torch.tensor([ms], dtype=torch.float64, device="cuda")
         dist.all_reduce(t, op=dist.ReduceOp.MAX)
         ms = float(t.item())
+    if args.dump_outputs and rank == 0:
+        dump_solve(args.dump_outputs, res)
     value = total_iters / (ms * 1e-3)
     fun = res.fun()
     n_loc_rank = rp.n

@@ -6,6 +6,9 @@ import os
 import subprocess
 import sys
 
+import numpy as np
+import pytest
+
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
 
@@ -63,3 +66,48 @@ def test_both_arms_share_one_config_dict():
         for world in (1, 8):
             c = bench.bench_config(wl, m, n, 0, world)
             assert set(c) == {"workload", "parallelism", "l2"} and wl in c["workload"]
+
+
+def _bench(*argv, timeout=120):
+    return subprocess.run([sys.executable, os.path.join(ROOT, "bench.py")] + list(argv), capture_output=True, text=True,
+                          timeout=timeout, cwd=ROOT)
+
+
+def test_steps_warmup_and_dump_outputs_are_validated(tmp_path):
+    for argv in (["--steps", "0"], ["--warmup", "-1"], ["--impl", "reference", "--dump-outputs", str(tmp_path / "d")]):
+        r = _bench(*argv)
+        assert r.returncode == 2 and "error:" in r.stderr, (argv, r.stderr[-2000:])
+    assert not (tmp_path / "d").exists()
+
+
+def test_dump_outputs_writes_float64_npy_within_the_limit(tmp_path):
+    sys.path.insert(0, ROOT)
+    import bench
+    bench.dump_outputs(str(tmp_path / "d"), {"x": np.arange(5, dtype=np.float32), "fun": -1.5, "iteration": 14})
+    got = {f: np.load(str(tmp_path / "d" / f)) for f in sorted(os.listdir(tmp_path / "d"))}
+    assert sorted(got) == ["fun.npy", "iteration.npy", "x.npy"]
+    assert all(a.dtype == np.float64 for a in got.values())
+    np.testing.assert_array_equal(got["x.npy"], np.arange(5.0))
+    assert got["fun.npy"] == -1.5 and got["iteration.npy"] == 14.0
+    with pytest.raises(ValueError):
+        bench.dump_outputs(str(tmp_path / "big"), {"x": np.zeros(bench.DUMP_LIMIT_BYTES // 8 + 1)})
+    assert not (tmp_path / "big").exists()
+
+
+@pytest.mark.gpu
+def test_dump_outputs_hold_the_last_timed_solve(tmp_path):
+    """The product arm on C1 (two timed solves): x, fun and iteration as a caller of `solve_resident` receives them,
+    within the parity bar of the committed oracle fixture."""
+    out = tmp_path / "out"
+    r = _bench("--workload", "C1", "--steps", "2", "--warmup", "1", "--no-cpu-baseline", "--no-e2e",
+               "--dump-outputs", str(out), timeout=600)
+    assert r.returncode == 0, r.stderr[-2000:]
+    d = json.loads([l for l in r.stdout.splitlines() if l.startswith("{")][0])
+    assert d["steps"] == 2 and d["warmup"] == 1
+    gold = json.load(open(os.path.join(ROOT, "tests", "golden", "oracle_C1_seed0.json")))
+    x = np.load(str(out / "x.npy"))
+    fun, it = float(np.load(str(out / "fun.npy"))), float(np.load(str(out / "iteration.npy")))
+    assert x.dtype == np.float64 and x.shape == (768,)
+    assert np.abs(x - np.load(os.path.join(ROOT, "tests", "golden", gold["x_file"]))).max() <= 1e-6
+    assert abs(it - gold["iterations"]) <= 1 and it == d["details"]["iterations_per_solve"]
+    assert abs(fun - gold["fun"]) <= 1e-8 * abs(gold["fun"]) and fun == d["details"]["objective"]

@@ -14,11 +14,14 @@ from lp_b200 import _ffi, api
 
 
 class _FakeLib:
-    """Stands in for liblpb200 in _HostBuffer: 'pinned' memory is a ctypes array we hold, frees are recorded."""
+    """Stands in for liblpb200 in _HostBuffer: 'pinned' memory is a ctypes array we hold, frees of it are recorded.
+    A free of any other address (real pinned memory of an earlier GPU test, collected while the fake is installed)
+    goes to the real library."""
 
     def __init__(self, real):
         self._real = real
         self.live = {}
+        self.allocated = set()
         self.freed = []
 
     def lpb_device_count(self):
@@ -28,11 +31,14 @@ class _FakeLib:
         mem = (C.c_ubyte * max(1, nbytes))()
         addr = C.addressof(mem)
         self.live[addr] = mem
+        self.allocated.add(addr)
         C.cast(pref, C.POINTER(C.c_void_p))[0] = addr
         return _ffi.LPB_OK
 
     def lpb_host_free(self, p):
         addr = p.value if hasattr(p, "value") else int(p)
+        if addr not in self.allocated:
+            return self._real.lpb_host_free(p)
         self.freed.append(addr)
         mem = self.live.pop(addr)
         C.memset(mem, 0xFF, len(mem))  # poison: a dangling view would read NaN patterns
