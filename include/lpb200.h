@@ -223,7 +223,16 @@ int lpb_extract_x(lpb_ctx* ctx, double tau, double* x_out, double* fun);
 int lpb_solve_batched(int64_t batch, int64_t m, int64_t n, const double* A, const double* b,
                       const double* c, const lpb_options* opts, double* x_out, double* fun,
                       int64_t* iterations, int32_t* status, int mem, void* stream);
-/* Free the device staging memory lpb_solve_batched keeps between calls with host inputs (per calling thread). */
+/* Same arguments and outputs as lpb_solve_batched, for 1 <= m <= 128.  The kernel follows from the shape: the
+ * shared-memory kernel of lpb_solve_batched (K6) where it accepts (m, n) -- m <= 64 and A beside M within 227 KB
+ * of shared memory, slack block not counted -- else K8, which reads A through L2 and keeps M and the vectors
+ * (about 80 n + 8 m^2 bytes; (128, 768) fits) in shared memory.  Other shapes: LPB_ERR_UNSUPPORTED, checked
+ * before any device is touched; lpb_last_error names the limit. */
+int lpb_solve_many(int64_t batch, int64_t m, int64_t n, const double* A, const double* b,
+                   const double* c, const lpb_options* opts, double* x_out, double* fun,
+                   int64_t* iterations, int32_t* status, int mem, void* stream);
+/* Free the device staging memory lpb_solve_batched / lpb_solve_many keep between calls with host inputs (per calling
+ * thread). */
 int lpb_release_workspaces(void);
 
 /* ------------------------------------------------------------------ kernel entry points

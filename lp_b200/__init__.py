@@ -11,6 +11,7 @@ from .api import (  # noqa: F401
     ShardedProblem,
     SyntheticShardedProblem,
     solve_batched,
+    solve_many,
     pinned_empty,
     presolve,
     Presolved,
@@ -33,7 +34,7 @@ from .api import (  # noqa: F401
 )
 
 __all__ = [
-    "BatchedResult", "ResidentProblem", "ShardedProblem", "SyntheticShardedProblem", "solve_batched", "pinned_empty", "presolve", "Presolved", "release_cached_contexts",
+    "BatchedResult", "ResidentProblem", "ShardedProblem", "SyntheticShardedProblem", "solve_batched", "solve_many", "pinned_empty", "presolve", "Presolved", "release_cached_contexts",
     "EquationSolverType", "IncompatibleInputDimensions", "Infeasible", "InteriorPoint", "InteriorPointBuilder",
     "InvalidParameter", "IterationLimitExceeded", "LinearProgramError", "NumericalProblem", "OptimizeResult",
     "Problem", "ProblemBuilder", "Solver", "Unbounded", "Unconstrained",

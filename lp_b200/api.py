@@ -480,16 +480,14 @@ class ResidentProblem:
 
 
 class BatchedResult:
-    """Outcome of `solve_batched`: per-problem x (user variables only), fun, iteration and status code
+    """Outcome of `solve_batched` / `solve_many`: per-problem x (user variables only), fun, iteration and status code
     (0 = Optimal, else the LPB_ERR_* code of the LinearProgramError variant)."""
 
     def __init__(self, x, x_slack, fun, iteration, status):
         self.x, self.x_slack, self.fun, self.iteration, self.status = x, x_slack, fun, iteration, status
 
 
-def solve_batched(A, b, c, n_slack: int = 0, solver: Optional["InteriorPoint"] = None, stream: int = 0):
-    """Solve `batch` independent slack-form LPs (A: batch x m x n, b: batch x m, c: batch x n) with one
-    CTA per problem (the whole solve_normal_form loop on device).  Host arrays in, host arrays out."""
+def _solve_batch(entry, A, b, c, n_slack, solver, stream):
     lib = _ffi.load()
     A = np.ascontiguousarray(A, dtype=np.float64)
     b = np.ascontiguousarray(b, dtype=np.float64)
@@ -502,11 +500,25 @@ def solve_batched(A, b, c, n_slack: int = 0, solver: Optional["InteriorPoint"] =
     fun = np.zeros(batch)
     it = np.zeros(batch, dtype=np.int64)
     st = np.zeros(batch, dtype=np.int32)
-    rc = lib.lpb_solve_batched(batch, m, n, A.ctypes.data, b.ctypes.data, c.ctypes.data, C.byref(solver._o),
-                               x.ctypes.data, fun.ctypes.data, it.ctypes.data, st.ctypes.data, _ffi.LPB_MEM_HOST,
-                               C.c_void_p(stream))
+    rc = getattr(lib, entry)(batch, m, n, A.ctypes.data, b.ctypes.data, c.ctypes.data, C.byref(solver._o),
+                             x.ctypes.data, fun.ctypes.data, it.ctypes.data, st.ctypes.data, _ffi.LPB_MEM_HOST,
+                             C.c_void_p(stream))
     _raise_for(rc)
     return BatchedResult(x[:, : n - n_slack].copy(), x, fun, it, st)
+
+
+def solve_batched(A, b, c, n_slack: int = 0, solver: Optional["InteriorPoint"] = None, stream: int = 0):
+    """Solve `batch` independent slack-form LPs (A: batch x m x n, b: batch x m, c: batch x n) with one
+    CTA per problem (the whole solve_normal_form loop on device).  Host arrays in, host arrays out."""
+    return _solve_batch("lpb_solve_batched", A, b, c, n_slack, solver, stream)
+
+
+def solve_many(A, b, c, n_slack: int = 0, solver: Optional["InteriorPoint"] = None, stream: int = 0):
+    """Like `solve_batched`, for LPs of up to 128 rows: problems of up to 64 rows whose A fits beside M in shared
+    memory run on `solve_batched`'s kernel, the others on one that reads A through L2.  n is limited by the shared
+    memory the rest of a problem needs (n = 768 fits at m = 128); a shape beyond the limits raises InvalidParameter
+    naming the limit."""
+    return _solve_batch("lpb_solve_many", A, b, c, n_slack, solver, stream)
 
 
 class Presolved:

@@ -1,24 +1,28 @@
-// batched.cu -- K6: many small independent LPs, one CTA per problem, the whole
+// batched.cu -- K6 / K8: many small independent LPs, one CTA per problem, the whole
 // solve_normal_form loop (interior_point/mod.rs:199-240) on the device.
 //
-// The CTA keeps A (m x n), M / L (m x m) and every iterate vector in shared memory and runs the
+// K6 (m <= 64) keeps A (m x n), M / L (m x m) and every iterate vector in shared memory; K8 (m <= 128) keeps A in
+// global memory and reads it through L2 (batched_streamed_kernel).  Both run the
 // SAME driver template as the single-problem path (ipm_driver.hpp: solve_normal_form_rec), here
-// instantiated on `SmemDev`, whose phase calls are block-cooperative device functions.  All 256
-// threads execute the scalar logic redundantly on block-broadcast reduction results, so control
+// instantiated on `SmemDev`, whose phase calls are block-cooperative device functions.  All threads
+// of the CTA execute the scalar logic redundantly on block-broadcast reduction results, so control
 // flow is uniform and the statuses / iteration counts follow the reference exactly like the
 // large-problem path does.  Problems are independent: sharding a batch over GPUs needs no collective.
 #include "ipm_driver.hpp"
 #include "kernels.hpp"
 #include "panel_factor.cuh"
 
+#include <type_traits>
+
 namespace lpb {
 namespace {
 
 constexpr int kBT = 256;       // threads per CTA
-constexpr int kBWarps = kBT / 32;
 constexpr int kMaxM = 64;      // register-tiled SYRK covers 64 x 64
 constexpr int kSB = 16;        // sub-block of the in-CTA blocked Cholesky
 constexpr int kXP = kSB + 1;   // pitch of the 16 x 16 inverted diagonal sub-blocks
+constexpr int kBT8 = 512;      // K8 (batched_streamed_kernel): 16 warps of 8 rows each for up to kMaxM8 rows
+constexpr int kMaxM8 = 128;
 
 __device__ __forceinline__ double bw_sum(double v) {
 #pragma unroll
@@ -31,36 +35,53 @@ __device__ __forceinline__ double bw_min(double v) {
   return v;
 }
 
-// Block all-reduce of NV values; every thread returns with the folded results (fixed order).
-template <int NV>
+// Block all-reduce of NV values over NW warps; every thread returns with the folded results (fixed order).
+template <int NW, int NV>
 __device__ __forceinline__ void block_allreduce(double (&v)[NV], const bool is_min, double* red) {
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
 #pragma unroll
   for (int k = 0; k < NV; ++k) {
     const double r = is_min ? bw_min(v[k]) : bw_sum(v[k]);
-    if (lane == 0) red[k * kBWarps + warp] = r;
+    if (lane == 0) red[k * NW + warp] = r;
   }
   __syncthreads();
 #pragma unroll
   for (int k = 0; k < NV; ++k) {
-    double r = red[k * kBWarps];
+    double r = red[k * NW];
 #pragma unroll
-    for (int w = 1; w < kBWarps; ++w) r = is_min ? fmin(r, red[k * kBWarps + w]) : r + red[k * kBWarps + w];
+    for (int w = 1; w < NW; ++w) r = is_min ? fmin(r, red[k * NW + w]) : r + red[k * NW + w];
     v[k] = r;
   }
   __syncthreads();
 }
 
+// The device side of the driver for one LP per CTA: MAXM rows at most, NT threads, A in shared memory (K6) or read
+// through L2 from global memory (A_GLOBAL, K8).  Everything else -- M / L, the inverted diagonal sub-blocks, every
+// vector -- lives in shared memory in both.
+template <int MAXM, int NT, bool A_GLOBAL>
 struct SmemDev {
+  static constexpr int kMaxM = MAXM;
+  static constexpr int kBT = NT;
+  static constexpr int kBWarps = NT / 32;
+  static constexpr bool kAGlobal = A_GLOBAL;
+  static_assert(kMaxM / kBWarps == 8, "rows_dot's transposing butterfly folds 8 rows per warp");
   int m, n, lda, ldm;
   int nd, ns;  // A holds the nd = n - ns leading columns; the ns trailing ones are the implicit identity block e_0 .. e_{ns-1}
   int mp, nsb;           // m rounded up to a multiple of 16 (rows >= m of M are identity padding), mp / 16
   double *Xinv, *cbuf;   // nsb x 16 x kXP inverted diagonal sub-blocks of L; scratch of factor_sub16 (panel_factor.cuh)
   int* flag;             // bad-pivot flag of the factorisation (shared)
-  double *A, *M, *b, *c, *x, *y, *z, *rP, *rD, *dinv, *xs, *r1, *p, *q, *u, *v, *dx, *dy, *dz, *t0, *t1, *sx,
-      *red;
+  const double* A;       // K6: shared, pitch batched_lda(nd); K8: this LP's rows in global memory, pitch n
+  double *M, *b, *c, *x, *y, *z, *rP, *rD, *dinv, *xs, *r1, *p, *q, *u, *v, *dx, *dy, *dz, *t0, *t1, *sx, *red;
   int have_pq, nan_pq;
   double cp, bq;
+
+  // A is read-only for the whole solve: from global memory through the non-coherent (read-only) path
+  __device__ __forceinline__ static double load_a(const double* p) {
+    if constexpr (A_GLOBAL)
+      return __ldg(p);
+    else
+      return *p;
+  }
 
   // t_k[i] = sum_j A[i][j] * (w_k[j] * (scale ? dinv[j] : 1)).  A warp owns the rows warp, warp + 8, ... (8 of them at
   // m = 64) and sums them TOGETHER: 8 accumulators per lane over its columns, then a transposing butterfly -- at offset
@@ -74,12 +95,15 @@ struct SmemDev {
     const unsigned full = 0xffffffffu;
     constexpr int R = kMaxM / kBWarps;  // 8 rows per warp
     double s0[R], s1[R];
-    const double* ar[R];
+    std::conditional_t<A_GLOBAL, int, const double*> ar[R];  // K8: 32-bit row offsets (pointers spill there)
 #pragma unroll
     for (int r = 0; r < R; ++r) {
       s0[r] = s1[r] = 0.0;
       const int row = warp + kBWarps * r;
-      ar[r] = A + (row < m ? row : 0) * lda;  // rows >= m: a valid row, result dropped
+      if constexpr (A_GLOBAL)
+        ar[r] = (row < m ? row : 0) * lda;
+      else
+        ar[r] = A + (row < m ? row : 0) * lda;  // rows >= m: a valid row, result dropped
     }
     for (int j = lane; j < nd; j += 32) {
       const double d = SCALE ? dinv[j] : 1.0;
@@ -87,7 +111,11 @@ struct SmemDev {
       const double x1 = NRHS == 2 ? (SCALE ? d * w1[j] : w1[j]) : 0.0;
 #pragma unroll
       for (int r = 0; r < R; ++r) {
-        const double a = ar[r][j];
+        double a;
+        if constexpr (A_GLOBAL)
+          a = __ldg(A + j + ar[r]);
+        else
+          a = ar[r][j];
         s0[r] += a * x0;
         if (NRHS == 2) s1[r] += a * x1;
       }
@@ -136,13 +164,13 @@ struct SmemDev {
     for (; i + 3 < m; i += 4) {
 #pragma unroll
       for (int e = 0; e < 4; ++e) {
-        const double a = col[(i + e) * lda];
+        const double a = load_a(col + (i + e) * lda);
         a0[e] += a * v0[i + e];
         if (NRHS == 2) a1[e] += a * v1[i + e];
       }
     }
     for (; i < m; ++i) {
-      const double a = col[i * lda];
+      const double a = load_a(col + i * lda);
       a0[0] += a * v0[i];
       if (NRHS == 2) a1[0] += a * v1[i];
     }
@@ -183,7 +211,7 @@ struct SmemDev {
       r[3] += rp * rp;
       r[4] += bi * y[i];
     }
-    block_allreduce<5>(r, false, red);
+    block_allreduce<kBWarps>(r, false, red);
     o->nrm_rd = sqrt(r[0]);
     o->cx = r[1];
     o->xz = r[2];
@@ -206,9 +234,10 @@ struct SmemDev {
       const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
       const int g = lane >> 2, t = lane & 3;
       const int nt = (m + 7) >> 3, ntiles = nt * (nt + 1) / 2;
-      constexpr int kTilesPerWarp = (kMaxM / 8) * (kMaxM / 8 + 1) / 2 / kBWarps + 1;  // 36 tiles / 8 warps -> 5
-      const double* ap[kTilesPerWarp];
-      const double* bp[kTilesPerWarp];
+      constexpr int kTilesPerWarp = (kMaxM / 8) * (kMaxM / 8 + 1) / 2 / kBWarps + 1;  // K6: 36 / 8 -> 5, K8: 136 / 16 -> 9
+      // K6: fragment pointers into shared memory; K8: 32-bit offsets of the tile rows from A (64-bit pointers spill there)
+      using Frag = std::conditional_t<A_GLOBAL, int, const double*>;
+      Frag ap[kTilesPerWarp], bp[kTilesPerWarp];
       int trow[kTilesPerWarp], tcol[kTilesPerWarp];
       double c0[kTilesPerWarp], c1[kTilesPerWarp];
 #pragma unroll
@@ -219,8 +248,13 @@ struct SmemDev {
         int bi = 0;
         while ((bi + 1) * (bi + 2) / 2 <= tile) ++bi;
         const int bj = tile - bi * (bi + 1) / 2;
-        ap[q] = A + (bi * 8 + g) * lda + t;
-        bp[q] = A + (bj * 8 + g) * lda + t;
+        if constexpr (A_GLOBAL) {  // rows >= m are clamped to a row of this LP: reading past it could leave the allocation
+          ap[q] = min(bi * 8 + g, m - 1) * lda;
+          bp[q] = min(bj * 8 + g, m - 1) * lda;
+        } else {
+          ap[q] = A + (bi * 8 + g) * lda + t;
+          bp[q] = A + (bj * 8 + g) * lda + t;
+        }
         trow[q] = live ? bi * 8 + g : m;  // m: nothing is stored
         tcol[q] = bj * 8 + 2 * t;
         c0[q] = c1[q] = 0.0;
@@ -229,12 +263,30 @@ struct SmemDev {
       // per LANE, each behind a predicated WARPSYNC.ALL -- a deadlock as soon as n is not a multiple of 4 (found the
       // hard way).  Instead the padding columns nd .. lda-1 of A are zero (written at load) and the index of dinv is
       // clamped, so the K tail contributes exact zeros.
+      // K8 reads A where the caller put it, so its columns past nd are not zeros: there the column index is clamped
+      // as well and the weight is multiplied by live = 0 (integer min / max, no predicate), which makes the K tail
+      // exact zeros for finite A.
       for (int k0 = 0; k0 < nd; k0 += 4) {
-        const double dk = dinv[min(k0 + t, nd - 1)];
+        double dk;
+        const double* ak;  // ap[q] / bp[q] are relative to it
+        if constexpr (A_GLOBAL) {
+          const int kc = min(k0 + t, nd - 1);
+          dk = dinv[kc] * (double)min(max(nd - (k0 + t), 0), 1);
+          ak = A + kc;
+        } else {
+          dk = dinv[min(k0 + t, nd - 1)];
+          ak = nullptr;
+        }
 #pragma unroll
         for (int q = 0; q < kTilesPerWarp; ++q) {
-          const double a = ap[q][k0];
-          const double bv = bp[q][k0] * dk;
+          double a, bv;
+          if constexpr (A_GLOBAL) {
+            a = __ldg(ak + ap[q]);
+            bv = __ldg(ak + bp[q]) * dk;
+          } else {
+            a = ap[q][k0];
+            bv = bp[q][k0] * dk;
+          }
           asm volatile("mma.sync.aligned.m8n8k4.row.col.f64.f64.f64.f64 {%0, %1}, {%2}, {%3}, {%0, %1};"
                        : "+d"(c0[q]), "+d"(c1[q])
                        : "d"(a), "d"(bv));
@@ -449,7 +501,7 @@ struct SmemDev {
         r[5] += (qi != qi) ? 1.0 : 0.0;
       }
     }
-    block_allreduce<6>(r, false, red);
+    block_allreduce<kBWarps>(r, false, red);
     if (with_pq) {
       cp = r[1];
       bq = r[4];
@@ -477,7 +529,7 @@ struct SmemDev {
       if (dzj < 0.0) r[1] = fmin(r[1], zj / -dzj);   // :62
     }
     for (int i = threadIdx.x; i < m; i += kBT) dy[i] = v[i] + q[i] * d_tau;  // delta.rs:34
-    block_allreduce<2>(r, true, red);
+    block_allreduce<kBWarps>(r, true, red);
     axz[0] = r[0];
     axz[1] = r[1];
     return LPB_OK;
@@ -499,14 +551,100 @@ struct SmemDev {
   }
 };
 
+using K6Dev = SmemDev<kMaxM, kBT, false>;
+using K8Dev = SmemDev<kMaxM8, kBT8, true>;
+
 __host__ __device__ inline int batched_mp(int m) { return (m + kSB - 1) / kSB * kSB; }
 // pitch of A in shared memory: = 4 (mod 16) doubles, so that the 8 x 4 DMMA fragment loads of the in-CTA SYRK (row g,
 // column t of a tile: 8 (g) + 2 (t) words apart) fall into 32 different banks per half-warp
 __host__ __device__ inline int batched_lda(int n) { return (n + 15) / 16 * 16 + 4; }
-__host__ __device__ inline size_t batched_smem_doubles(int m, int n, int ns) {
+// everything but A (the only term of K6's footprint that K8 does not have)
+template <class Dev>
+__host__ __device__ inline size_t batched_vec_smem_doubles(int m, int n) {
   const size_t mp = (size_t)batched_mp(m);
-  return (size_t)m * batched_lda(n - ns) + mp * (mp + 1) + 10 * (size_t)n + 5 * (size_t)m + 2 * mp + 2 * kMaxM + 8 * kBWarps +
+  return mp * (mp + 1) + 10 * (size_t)n + 5 * (size_t)m + 2 * mp + 2 * Dev::kMaxM + 8 * Dev::kBWarps +
          (mp / kSB) * kSB * kXP + panel_factor_scratch(kXP) + 2;
+}
+__host__ __device__ inline size_t batched_smem_doubles(int m, int n, int ns) {
+  return (size_t)m * batched_lda(n - ns) + batched_vec_smem_doubles<K6Dev>(m, n);
+}
+
+// Layout of everything behind A in the dynamic shared memory (the same for K6 and K8).
+template <class Dev>
+__device__ __forceinline__ void carve_smem(Dev& d, double* ptr) {
+  auto take = [&](size_t cnt) {
+    double* r = ptr;
+    ptr += cnt;
+    return r;
+  };
+  d.M = take((size_t)d.mp * d.ldm);
+  d.c = take(d.n); d.x = take(d.n); d.z = take(d.n); d.rD = take(d.n); d.dinv = take(d.n); d.xs = take(d.n);
+  d.r1 = take(d.n); d.p = take(d.n); d.dx = take(d.n); d.dz = take(d.n);
+  d.u = d.r1;        // u[j] = dinv[j] * (s - r1[j]) overwrites r1[j] in place (r1 is dead afterwards)
+  d.b = take(d.m); d.y = take(d.m); d.rP = take(d.m); d.q = take(d.mp); d.v = take(d.mp); d.dy = take(d.m);
+  d.t0 = take(d.m);
+  d.t1 = d.dy;       // t1 is consumed (q = b + t1) before d_y is written
+  d.sx = take(2 * Dev::kMaxM);
+  d.red = take(8 * Dev::kBWarps);
+  d.Xinv = take((size_t)d.nsb * kSB * kXP);
+  d.cbuf = take(panel_factor_scratch(kXP));
+  d.flag = reinterpret_cast<int*>(take(2));
+  d.have_pq = 0;
+  d.nan_pq = 0;
+  d.cp = d.bq = 0.0;
+}
+
+template <class Dev>
+__device__ __forceinline__ void init_dims(Dev& d, int m, int n, int ns) {
+  d.m = m;
+  d.n = n;
+  d.ns = ns;
+  d.nd = n - ns;
+  d.lda = Dev::kAGlobal ? n : batched_lda(d.nd);
+  d.mp = batched_mp(m);
+  d.nsb = d.mp / kSB;
+  d.ldm = d.mp + 1;
+}
+
+// Loads the rest of problem `lp` (A is in place), runs the driver and writes its outputs.
+template <class Dev>
+__device__ __forceinline__ void solve_one(Dev& d, int64_t lp, const double* __restrict__ gb,
+                                          const double* __restrict__ gc, const lpb_options& opts,
+                                          double* __restrict__ x_out, double* __restrict__ fun_out,
+                                          int64_t* __restrict__ it_out, int32_t* __restrict__ st_out) {
+  constexpr int kT = Dev::kBT;
+  const int m = d.m, n = d.n;
+  for (int idx = threadIdx.x; idx < d.mp * d.mp; idx += kT) {  // identity padding of M beyond m (kept by the factorisation)
+    const int r = idx / d.mp, cc = idx - r * d.mp;
+    if (r >= m || cc >= m) d.M[r * d.ldm + cc] = (r == cc) ? 1.0 : 0.0;
+  }
+  for (int i = threadIdx.x; i < m; i += kT) d.b[i] = gb[lp * m + i];
+  for (int j = threadIdx.x; j < n; j += kT) {
+    d.c[j] = gc[lp * n + j];
+    d.dx[j] = 0.0;
+    d.dz[j] = 0.0;
+  }
+  __syncthreads();
+
+  SolveScalars sc;
+  NullRecorder rec;
+  const int rc = solve_normal_form_rec(d, opts, (int64_t)n, 0.0, &sc, rec);
+
+  double f[1] = {0.0};
+  if (rc == LPB_OK || rc == LPB_ERR_ITERATION_LIMIT_EXCEEDED) {
+    for (int j = threadIdx.x; j < n; j += kT) {
+      const double t = d.x[j] / sc.tau;  // mod.rs:231
+      x_out[lp * n + j] = t;
+      f[0] += d.c[j] * t;                // linear_program.rs:62
+    }
+  }
+  block_allreduce<Dev::kBWarps>(f, false, d.red);
+  if (threadIdx.x == 0) {
+    fun_out[lp] = f[0];
+    it_out[lp] = sc.iterations;
+    st_out[lp] = rc;
+  }
+  __syncthreads();
 }
 
 // Two CTAs per SM (128 registers, <= 113 KB of shared memory each) whenever the batch has the slack structure: one LP's
@@ -519,78 +657,41 @@ batched_ipm_kernel(int64_t batch, int m, int n, int ns, const double* __restrict
                    double* __restrict__ fun_out, int64_t* __restrict__ it_out, int32_t* __restrict__ st_out) {
   extern __shared__ double sm[];
   for (int64_t lp = blockIdx.x; lp < batch; lp += gridDim.x) {
-    SmemDev d;
-    d.m = m;
-    d.n = n;
-    d.ns = ns;
-    d.nd = n - ns;
-    d.lda = batched_lda(d.nd);
-    d.mp = batched_mp(m);
-    d.nsb = d.mp / kSB;
-    d.ldm = d.mp + 1;
-    double* ptr = sm;
-    auto take = [&](size_t cnt) {
-      double* r = ptr;
-      ptr += cnt;
-      return r;
-    };
-    d.A = take((size_t)m * d.lda);
-    d.M = take((size_t)d.mp * d.ldm);
-    d.c = take(n); d.x = take(n); d.z = take(n); d.rD = take(n); d.dinv = take(n); d.xs = take(n);
-    d.r1 = take(n); d.p = take(n); d.dx = take(n); d.dz = take(n);
-    d.u = d.r1;        // u[j] = dinv[j] * (s - r1[j]) overwrites r1[j] in place (r1 is dead afterwards)
-    d.b = take(m); d.y = take(m); d.rP = take(m); d.q = take(d.mp); d.v = take(d.mp); d.dy = take(m);
-    d.t0 = take(m);
-    d.t1 = d.dy;       // t1 is consumed (q = b + t1) before d_y is written
-    d.sx = take(2 * kMaxM);
-    d.red = take(8 * kBWarps);
-    d.Xinv = take((size_t)d.nsb * kSB * kXP);
-    d.cbuf = take(panel_factor_scratch(kXP));
-    d.flag = reinterpret_cast<int*>(take(2));
-    d.have_pq = 0;
-    d.nan_pq = 0;
-    d.cp = d.bq = 0.0;
+    K6Dev d;
+    init_dims(d, m, n, ns);
+    double* sA = sm;
+    d.A = sA;
+    carve_smem(d, sm + (size_t)m * d.lda);
 
     const double* A = gA + lp * (int64_t)m * n;
     for (int idx = threadIdx.x; idx < m * d.nd; idx += kBT) {
       const int i = idx / d.nd, j = idx - i * d.nd;
-      d.A[i * d.lda + j] = A[i * n + j];
+      sA[i * d.lda + j] = A[i * n + j];
     }
     for (int idx = threadIdx.x; idx < m * (d.lda - d.nd); idx += kBT) {  // zero padding columns: the K tail of the DMMA SYRK
       const int i = idx / (d.lda - d.nd), j = d.nd + idx - i * (d.lda - d.nd);
-      d.A[i * d.lda + j] = 0.0;
+      sA[i * d.lda + j] = 0.0;
     }
-    for (int idx = threadIdx.x; idx < d.mp * d.mp; idx += kBT) {  // identity padding of M beyond m (kept by the factorisation)
-      const int r = idx / d.mp, cc = idx - r * d.mp;
-      if (r >= m || cc >= m) d.M[r * d.ldm + cc] = (r == cc) ? 1.0 : 0.0;
-    }
-    for (int i = threadIdx.x; i < m; i += kBT) d.b[i] = gb[lp * m + i];
-    for (int j = threadIdx.x; j < n; j += kBT) {
-      d.c[j] = gc[lp * n + j];
-      d.dx[j] = 0.0;
-      d.dz[j] = 0.0;
-    }
-    __syncthreads();
+    solve_one(d, lp, gb, gc, opts, x_out, fun_out, it_out, st_out);
+  }
+}
 
-    SolveScalars sc;
-    NullRecorder rec;
-    const int rc = solve_normal_form_rec(d, opts, (int64_t)n, 0.0, &sc, rec);
-
-    double f[1] = {0.0};
-    if (rc == LPB_OK || rc == LPB_ERR_ITERATION_LIMIT_EXCEEDED) {
-      for (int j = threadIdx.x; j < n; j += kBT) {
-        const double t = d.x[j] / sc.tau;  // mod.rs:231
-        x_out[lp * n + j] = t;
-        f[0] += d.c[j] * t;                // linear_program.rs:62
-      }
-    }
-    block_allreduce<1>(f, false, d.red);
-    if (threadIdx.x == 0) {
-      fun_out[lp] = f[0];
-      it_out[lp] = sc.iterations;
-      st_out[lp] = rc;
-    }
-    __syncthreads();
+// K8: LPs of up to 128 rows.  A (m x n, 128 x 256 = 256 KB) no longer fits beside M, so it stays in global memory and
+// every pass over it -- the SYRK, the row sweeps, the column sweeps -- reads it through L2 (148 resident LPs of
+// 128 x 128 dense columns are ~19 MB); the shared memory holds M / L and the vectors.  One CTA of 16 warps per SM:
+// rows_dot's 8 rows per warp then cover 128 rows, and chol_solve's thread-per-row layout covers both right-hand sides.
+__global__ void __launch_bounds__(kBT8, 1)
+batched_streamed_kernel(int64_t batch, int m, int n, int ns, const double* __restrict__ gA,
+                        const double* __restrict__ gb, const double* __restrict__ gc, lpb_options opts,
+                        double* __restrict__ x_out, double* __restrict__ fun_out, int64_t* __restrict__ it_out,
+                        int32_t* __restrict__ st_out) {
+  extern __shared__ double sm[];
+  for (int64_t lp = blockIdx.x; lp < batch; lp += gridDim.x) {
+    K8Dev d;
+    init_dims(d, m, n, ns);
+    d.A = gA + lp * (int64_t)m * n;
+    carve_smem(d, sm);
+    solve_one(d, lp, gb, gc, opts, x_out, fun_out, it_out, st_out);
   }
 }
 
@@ -600,7 +701,7 @@ batched_ipm_kernel(int64_t batch, int m, int n, int ns, const double* __restrict
 // consistent ns_lp), the batch takes the minimum.  A batch without the structure gets 0 and the kernel stores all of A.
 __global__ void __launch_bounds__(256)
 batched_structure_kernel(int64_t batch, int m, int n, const double* __restrict__ gA, int* __restrict__ ns_out) {
-  __shared__ int urow[kMaxM];  // urow[t]: column n - smax + t is the unit vector e_{urow[t]} (entry exactly 1), else -1
+  __shared__ int urow[kMaxM8];  // urow[t]: column n - smax + t is the unit vector e_{urow[t]} (entry exactly 1), else -1
   __shared__ int best;
   const int smax = m < n ? m : n;
   for (int64_t lp = blockIdx.x; lp < batch; lp += gridDim.x) {
@@ -629,13 +730,12 @@ batched_structure_kernel(int64_t batch, int m, int n, const double* __restrict__
 
 }  // namespace
 
-int batched_launch(int64_t batch, int m, int n, const double* dA, const double* db, const double* dc,
-                   const lpb_options& o, double* dx, double* dfun, int64_t* dit, int32_t* dst, cudaStream_t stream) {
-  if (m > kMaxM) {
-    set_last_error("solve_batched: needs m <= %d", kMaxM);
-    return LPB_ERR_UNSUPPORTED;
-  }
-  // structure scan: dit (int64 per problem, written by the solve afterwards) lends its first word for the result
+namespace {
+constexpr size_t kSmemCap = 227 * 1024;
+
+// Structure scan (batched_structure_kernel): dit (int64 per problem, written by the solve afterwards) lends its first
+// word for the result.
+int scan_slack_structure(int64_t batch, int m, int n, const double* dA, int64_t* dit, cudaStream_t stream, int* ns_out) {
   int* ns_dev = reinterpret_cast<int*>(dit);
   int ns = m < n ? m : n;
   LPB_CUDA(cudaMemcpyAsync(ns_dev, &ns, sizeof(int), cudaMemcpyHostToDevice, stream));
@@ -645,14 +745,67 @@ int batched_launch(int64_t batch, int m, int n, const double* dA, const double* 
   LPB_CUDA(cudaMemcpyAsync(&ns, ns_dev, sizeof(int), cudaMemcpyDeviceToHost, stream));
   LPB_CUDA(cudaStreamSynchronize(stream));
   if (ns < 0 || ns > m || ns >= n) ns = 0;
+  *ns_out = ns;
+  return LPB_OK;
+}
+
+int launch_k6(int64_t batch, int m, int n, int ns, const double* dA, const double* db, const double* dc,
+              const lpb_options& o, double* dx, double* dfun, int64_t* dit, int32_t* dst, cudaStream_t stream) {
   const size_t smem = batched_smem_doubles(m, n, ns) * sizeof(double);
-  if (smem > 227 * 1024) {
-    set_last_error("solve_batched: %zu bytes of shared memory > 227 KB", smem);
-    return LPB_ERR_UNSUPPORTED;
-  }
   LPB_CUDA(cudaFuncSetAttribute(batched_ipm_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
   const int64_t grid = batch < (int64_t)kNumSMs * 64 ? batch : (int64_t)kNumSMs * 64;
   batched_ipm_kernel<<<(unsigned)grid, kBT, smem, stream>>>(batch, m, n, ns, dA, db, dc, o, dx, dfun, dit, dst);
+  LPB_CUDA(cudaGetLastError());
+  return LPB_OK;
+}
+}  // namespace
+
+int batched_launch(int64_t batch, int m, int n, const double* dA, const double* db, const double* dc,
+                   const lpb_options& o, double* dx, double* dfun, int64_t* dit, int32_t* dst, cudaStream_t stream) {
+  if (m > kMaxM) {
+    set_last_error("solve_batched: needs m <= %d", kMaxM);
+    return LPB_ERR_UNSUPPORTED;
+  }
+  int ns = 0;
+  LPB_TRY(scan_slack_structure(batch, m, n, dA, dit, stream, &ns));
+  const size_t smem = batched_smem_doubles(m, n, ns) * sizeof(double);
+  if (smem > kSmemCap) {
+    set_last_error("solve_batched: %zu bytes of shared memory > 227 KB", smem);
+    return LPB_ERR_UNSUPPORTED;
+  }
+  return launch_k6(batch, m, n, ns, dA, db, dc, o, dx, dfun, dit, dst, stream);
+}
+
+// K8's footprint does not depend on the slack structure, and K6 fits wherever K8 does not only if K8 fits too: the
+// shape alone decides whether solve_many can run it, before any device is touched.
+int solve_many_check_shape(int64_t m, int64_t n) {
+  if (m > kMaxM8) {
+    set_last_error("solve_many: needs m <= %d (got m = %lld)", kMaxM8, (long long)m);
+    return LPB_ERR_UNSUPPORTED;
+  }
+  // n beyond 2^20 is far past the limit; the clamp keeps the count in int
+  const size_t smem = batched_vec_smem_doubles<K8Dev>((int)m, (int)(n < (1 << 20) ? n : (1 << 20))) * sizeof(double);
+  if (smem > kSmemCap) {
+    set_last_error("solve_many: m = %lld, n = %lld needs %zu bytes of shared memory > 227 KB (232448 bytes)",
+                   (long long)m, (long long)n, smem);
+    return LPB_ERR_UNSUPPORTED;
+  }
+  return LPB_OK;
+}
+
+// K6 where it accepts (m, n, ns) -- m <= 64 and A fits beside M -- else K8.  Which of the two is faster where both
+// run has not been measured: this only picks a kernel that can run the shape.
+int solve_many_launch(int64_t batch, int m, int n, const double* dA, const double* db, const double* dc,
+                      const lpb_options& o, double* dx, double* dfun, int64_t* dit, int32_t* dst, cudaStream_t stream) {
+  LPB_TRY(solve_many_check_shape(m, n));
+  int ns = 0;
+  LPB_TRY(scan_slack_structure(batch, m, n, dA, dit, stream, &ns));
+  if (m <= kMaxM && batched_smem_doubles(m, n, ns) * sizeof(double) <= kSmemCap)
+    return launch_k6(batch, m, n, ns, dA, db, dc, o, dx, dfun, dit, dst, stream);
+  const size_t smem = batched_vec_smem_doubles<K8Dev>(m, n) * sizeof(double);
+  LPB_CUDA(cudaFuncSetAttribute(batched_streamed_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
+  const int64_t grid = batch < (int64_t)kNumSMs * 64 ? batch : (int64_t)kNumSMs * 64;
+  batched_streamed_kernel<<<(unsigned)grid, kBT8, smem, stream>>>(batch, m, n, ns, dA, db, dc, o, dx, dfun, dit, dst);
   LPB_CUDA(cudaGetLastError());
   return LPB_OK;
 }

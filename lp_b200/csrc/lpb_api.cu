@@ -25,6 +25,9 @@ namespace lpb {
 int64_t gemv_t_partials_doubles(int64_t m, int64_t n);
 int batched_launch(int64_t batch, int m, int n, const double* dA, const double* db, const double* dc,
                    const lpb_options& o, double* dx, double* dfun, int64_t* dit, int32_t* dst, cudaStream_t stream);
+int solve_many_check_shape(int64_t m, int64_t n);
+int solve_many_launch(int64_t batch, int m, int n, const double* dA, const double* db, const double* dc,
+                      const lpb_options& o, double* dx, double* dfun, int64_t* dit, int32_t* dst, cudaStream_t stream);
 }
 
 using namespace lpb;
@@ -167,9 +170,9 @@ struct ProcessComm {
 ProcessComm g_comm;
 std::mutex g_comm_mu;
 
-// device staging arena of lpb_solve_batched for host inputs (per host thread, grow-only)
+// device staging arena of lpb_solve_batched / lpb_solve_many for host inputs (per host thread, grow-only)
 thread_local void* g_batched_ws = nullptr;
-thread_local cudaStream_t g_batched_copy_stream = nullptr;  // uploads of lpb_solve_batched (host inputs), see there
+thread_local cudaStream_t g_batched_copy_stream = nullptr;  // uploads of host inputs, see run_batched
 thread_local cudaEvent_t g_batched_ev[4] = {nullptr, nullptr, nullptr, nullptr};
 thread_local size_t g_batched_ws_cap = 0;
 
@@ -775,6 +778,93 @@ int need_problem(lpb_ctx* c) {
   return LPB_OK;
 }
 
+using BatchedLaunch = int (*)(int64_t, int, int, const double*, const double*, const double*, const lpb_options&, double*,
+                              double*, int64_t*, int32_t*, cudaStream_t);
+
+// Runs `launch` (K6 alone, or solve_many's choice) over the batch: directly on device arrays, or with host arrays staged
+// through the per-thread arena.
+int run_batched(BatchedLaunch launch, int64_t batch, int64_t m, int64_t n, const double* A, const double* b, const double* c,
+                const lpb_options& o, double* x_out, double* fun, int64_t* iterations, int32_t* status, int mem,
+                cudaStream_t st) {
+  if (mem == LPB_MEM_DEVICE) {
+    LPB_TRY(launch(batch, (int)m, (int)n, A, b, c, o, x_out, fun, iterations, status, st));
+    LPB_CUDA(cudaStreamSynchronize(st));
+    return LPB_OK;
+  }
+  // Host arrays: stage through ONE cached device arena per host thread (grow-only; lpb_release_workspaces
+  // frees it), so a call costs the three uploads, the kernel and the four downloads -- no cudaMalloc / cudaFree.
+  const size_t sA = sizeof(double) * (size_t)(batch * m * n), sb = sizeof(double) * (size_t)(batch * m),
+               sc = sizeof(double) * (size_t)(batch * n), s8 = sizeof(double) * (size_t)batch,
+               s4 = sizeof(int32_t) * (size_t)batch;
+  auto up = [](size_t v) { return (v + 255) & ~(size_t)255; };
+  const size_t need = up(sA) + up(sb) + 2 * up(sc) + 2 * up(s8) + up(s4);
+  if (g_batched_ws_cap < need) {
+    if (g_batched_ws) cudaFree(g_batched_ws);
+    g_batched_ws = nullptr;
+    g_batched_ws_cap = 0;
+    LPB_CUDA(cudaMalloc(&g_batched_ws, need));
+    g_batched_ws_cap = need;
+  }
+  char* p = static_cast<char*>(g_batched_ws);
+  auto carve = [&](size_t bytes) {
+    char* r = p;
+    p += up(bytes);
+    return r;
+  };
+  double* dA = reinterpret_cast<double*>(carve(sA));
+  double* db = reinterpret_cast<double*>(carve(sb));
+  double* dc = reinterpret_cast<double*>(carve(sc));
+  double* dx = reinterpret_cast<double*>(carve(sc));
+  double* df = reinterpret_cast<double*>(carve(s8));
+  int64_t* dit = reinterpret_cast<int64_t*>(carve(s8));
+  int32_t* dst = reinterpret_cast<int32_t*>(carve(s4));
+  // The batch goes through in chunks: all uploads are queued on a copy stream up front, chunk i's kernel waits for its
+  // own upload only, so the upload of chunk i + 1 (PCIe) runs under the kernel of chunk i and the downloads of chunk
+  // i - 1.  At C4 the upload (558 MB, ~10 ms from pinned memory) and the kernel (~11 ms) used to add up.
+  const int64_t nchunk = batch >= 1024 ? 4 : 1;
+  if (!g_batched_copy_stream) LPB_CUDA(cudaStreamCreateWithFlags(&g_batched_copy_stream, cudaStreamNonBlocking));
+  for (int q = 0; q < 4; ++q)
+    if (!g_batched_ev[q]) LPB_CUDA(cudaEventCreateWithFlags(&g_batched_ev[q], cudaEventDisableTiming));
+  LPB_CUDA(cudaEventRecord(g_batched_ev[0], st));  // the copy stream starts behind whatever `st` holds already
+  LPB_CUDA(cudaStreamWaitEvent(g_batched_copy_stream, g_batched_ev[0], 0));
+  auto lo = [&](int64_t q) { return batch * q / nchunk; };
+  for (int64_t q = 0; q < nchunk; ++q) {
+    const int64_t b0 = lo(q), nb = lo(q + 1) - b0;
+    LPB_CUDA(cudaMemcpyAsync(dA + b0 * m * n, A + b0 * m * n, sizeof(double) * (size_t)(nb * m * n), cudaMemcpyHostToDevice,
+                             g_batched_copy_stream));
+    LPB_CUDA(cudaMemcpyAsync(db + b0 * m, b + b0 * m, sizeof(double) * (size_t)(nb * m), cudaMemcpyHostToDevice,
+                             g_batched_copy_stream));
+    LPB_CUDA(cudaMemcpyAsync(dc + b0 * n, c + b0 * n, sizeof(double) * (size_t)(nb * n), cudaMemcpyHostToDevice,
+                             g_batched_copy_stream));
+    LPB_CUDA(cudaEventRecord(g_batched_ev[q], g_batched_copy_stream));
+  }
+  for (int64_t q = 0; q < nchunk; ++q) {
+    const int64_t b0 = lo(q), nb = lo(q + 1) - b0;
+    LPB_CUDA(cudaStreamWaitEvent(st, g_batched_ev[q], 0));
+    LPB_TRY(launch(nb, (int)m, (int)n, dA + b0 * m * n, db + b0 * m, dc + b0 * n, o, dx + b0 * n, df + b0, dit + b0,
+                   dst + b0, st));
+    LPB_CUDA(cudaMemcpyAsync(x_out + b0 * n, dx + b0 * n, sizeof(double) * (size_t)(nb * n), cudaMemcpyDeviceToHost, st));
+    LPB_CUDA(cudaMemcpyAsync(fun + b0, df + b0, sizeof(double) * (size_t)nb, cudaMemcpyDeviceToHost, st));
+    LPB_CUDA(cudaMemcpyAsync(iterations + b0, dit + b0, sizeof(int64_t) * (size_t)nb, cudaMemcpyDeviceToHost, st));
+    LPB_CUDA(cudaMemcpyAsync(status + b0, dst + b0, sizeof(int32_t) * (size_t)nb, cudaMemcpyDeviceToHost, st));
+  }
+  LPB_CUDA(cudaStreamSynchronize(st));
+  return LPB_OK;
+}
+
+int batched_args(const char* who, int64_t batch, int64_t m, int64_t n, const double* A, const double* b, const double* c,
+                 const lpb_options* opts, double* x_out, double* fun, int64_t* iterations, int32_t* status,
+                 lpb_options* o) {
+  if (batch <= 0 || m <= 0 || n <= 0 || !A || !b || !c || !x_out || !fun || !iterations || !status) {
+    set_last_error("%s: null pointer or non-positive size", who);
+    return LPB_ERR_BAD_ARGUMENT;
+  }
+  if (opts)
+    *o = *opts;
+  else
+    options_default(o);
+  return lpb_options_validate(o);
+}
 }  // namespace
 
 // ====================================================================== extern "C"
@@ -1292,82 +1382,22 @@ int lpb_k_gemv_t(lpb_ctx* c, int64_t m, int64_t n, const double* dA, int64_t lda
 int lpb_solve_batched(int64_t batch, int64_t m, int64_t n, const double* A, const double* b, const double* c,
                       const lpb_options* opts, double* x_out, double* fun, int64_t* iterations, int32_t* status,
                       int mem, void* stream) {
-  if (batch <= 0 || m <= 0 || n <= 0 || !A || !b || !c || !x_out || !fun || !iterations || !status) {
-    set_last_error("solve_batched: null pointer or non-positive size");
-    return LPB_ERR_BAD_ARGUMENT;
-  }
   lpb_options o;
-  if (opts)
-    o = *opts;
-  else
-    options_default(&o);
-  LPB_TRY(lpb_options_validate(&o));
+  LPB_TRY(batched_args("solve_batched", batch, m, n, A, b, c, opts, x_out, fun, iterations, status, &o));
   LPB_TRY(check_device());
-  cudaStream_t st = static_cast<cudaStream_t>(stream);
-  if (mem == LPB_MEM_DEVICE) {
-    LPB_TRY(batched_launch(batch, (int)m, (int)n, A, b, c, o, x_out, fun, iterations, status, st));
-    LPB_CUDA(cudaStreamSynchronize(st));
-    return LPB_OK;
-  }
-  // Host arrays: stage through ONE cached device arena per host thread (grow-only; lpb_release_workspaces
-  // frees it), so a call costs the three uploads, the kernel and the four downloads -- no cudaMalloc / cudaFree.
-  const size_t sA = sizeof(double) * (size_t)(batch * m * n), sb = sizeof(double) * (size_t)(batch * m),
-               sc = sizeof(double) * (size_t)(batch * n), s8 = sizeof(double) * (size_t)batch,
-               s4 = sizeof(int32_t) * (size_t)batch;
-  auto up = [](size_t v) { return (v + 255) & ~(size_t)255; };
-  const size_t need = up(sA) + up(sb) + 2 * up(sc) + 2 * up(s8) + up(s4);
-  if (g_batched_ws_cap < need) {
-    if (g_batched_ws) cudaFree(g_batched_ws);
-    g_batched_ws = nullptr;
-    g_batched_ws_cap = 0;
-    LPB_CUDA(cudaMalloc(&g_batched_ws, need));
-    g_batched_ws_cap = need;
-  }
-  char* p = static_cast<char*>(g_batched_ws);
-  auto carve = [&](size_t bytes) {
-    char* r = p;
-    p += up(bytes);
-    return r;
-  };
-  double* dA = reinterpret_cast<double*>(carve(sA));
-  double* db = reinterpret_cast<double*>(carve(sb));
-  double* dc = reinterpret_cast<double*>(carve(sc));
-  double* dx = reinterpret_cast<double*>(carve(sc));
-  double* df = reinterpret_cast<double*>(carve(s8));
-  int64_t* dit = reinterpret_cast<int64_t*>(carve(s8));
-  int32_t* dst = reinterpret_cast<int32_t*>(carve(s4));
-  // The batch goes through in chunks: all uploads are queued on a copy stream up front, chunk i's kernel waits for its
-  // own upload only, so the upload of chunk i + 1 (PCIe) runs under the kernel of chunk i and the downloads of chunk
-  // i - 1.  At C4 the upload (558 MB, ~10 ms from pinned memory) and the kernel (~11 ms) used to add up.
-  const int64_t nchunk = batch >= 1024 ? 4 : 1;
-  if (!g_batched_copy_stream) LPB_CUDA(cudaStreamCreateWithFlags(&g_batched_copy_stream, cudaStreamNonBlocking));
-  for (int q = 0; q < 4; ++q)
-    if (!g_batched_ev[q]) LPB_CUDA(cudaEventCreateWithFlags(&g_batched_ev[q], cudaEventDisableTiming));
-  LPB_CUDA(cudaEventRecord(g_batched_ev[0], st));  // the copy stream starts behind whatever `st` holds already
-  LPB_CUDA(cudaStreamWaitEvent(g_batched_copy_stream, g_batched_ev[0], 0));
-  auto lo = [&](int64_t q) { return batch * q / nchunk; };
-  for (int64_t q = 0; q < nchunk; ++q) {
-    const int64_t b0 = lo(q), nb = lo(q + 1) - b0;
-    LPB_CUDA(cudaMemcpyAsync(dA + b0 * m * n, A + b0 * m * n, sizeof(double) * (size_t)(nb * m * n), cudaMemcpyHostToDevice,
-                             g_batched_copy_stream));
-    LPB_CUDA(cudaMemcpyAsync(db + b0 * m, b + b0 * m, sizeof(double) * (size_t)(nb * m), cudaMemcpyHostToDevice,
-                             g_batched_copy_stream));
-    LPB_CUDA(cudaMemcpyAsync(dc + b0 * n, c + b0 * n, sizeof(double) * (size_t)(nb * n), cudaMemcpyHostToDevice,
-                             g_batched_copy_stream));
-    LPB_CUDA(cudaEventRecord(g_batched_ev[q], g_batched_copy_stream));
-  }
-  for (int64_t q = 0; q < nchunk; ++q) {
-    const int64_t b0 = lo(q), nb = lo(q + 1) - b0;
-    LPB_CUDA(cudaStreamWaitEvent(st, g_batched_ev[q], 0));
-    LPB_TRY(batched_launch(nb, (int)m, (int)n, dA + b0 * m * n, db + b0 * m, dc + b0 * n, o, dx + b0 * n, df + b0, dit + b0,
-                           dst + b0, st));
-    LPB_CUDA(cudaMemcpyAsync(x_out + b0 * n, dx + b0 * n, sizeof(double) * (size_t)(nb * n), cudaMemcpyDeviceToHost, st));
-    LPB_CUDA(cudaMemcpyAsync(fun + b0, df + b0, sizeof(double) * (size_t)nb, cudaMemcpyDeviceToHost, st));
-    LPB_CUDA(cudaMemcpyAsync(iterations + b0, dit + b0, sizeof(int64_t) * (size_t)nb, cudaMemcpyDeviceToHost, st));
-    LPB_CUDA(cudaMemcpyAsync(status + b0, dst + b0, sizeof(int32_t) * (size_t)nb, cudaMemcpyDeviceToHost, st));
-  }
-  LPB_CUDA(cudaStreamSynchronize(st));
-  return LPB_OK;
+  return run_batched(batched_launch, batch, m, n, A, b, c, o, x_out, fun, iterations, status, mem,
+                     static_cast<cudaStream_t>(stream));
+}
+
+int lpb_solve_many(int64_t batch, int64_t m, int64_t n, const double* A, const double* b, const double* c,
+                   const lpb_options* opts, double* x_out, double* fun, int64_t* iterations, int32_t* status, int mem,
+                   void* stream) {
+  lpb_options o;
+  LPB_TRY(batched_args("solve_many", batch, m, n, A, b, c, opts, x_out, fun, iterations, status, &o));
+  LPB_TRY(solve_many_check_shape(m, n));  // shape limits first: they hold or fail without a device
+  LPB_TRY(check_device());
+  return run_batched(solve_many_launch, batch, m, n, A, b, c, o, x_out, fun, iterations, status, mem,
+                     static_cast<cudaStream_t>(stream));
 }
 
 int lpb_release_workspaces(void) {
