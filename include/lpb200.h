@@ -231,8 +231,24 @@ int lpb_solve_batched(int64_t batch, int64_t m, int64_t n, const double* A, cons
 int lpb_solve_many(int64_t batch, int64_t m, int64_t n, const double* A, const double* b,
                    const double* c, const lpb_options* opts, double* x_out, double* fun,
                    int64_t* iterations, int32_t* status, int mem, void* stream);
-/* Free the device staging memory lpb_solve_batched / lpb_solve_many keep between calls with host inputs (per calling
- * thread). */
+/* lpb_solve_many's shape limits for one LP of m x n, on the host: LPB_OK if lpb_solve_many (and
+ * lpb_solve_many_ragged) can run the shape, LPB_ERR_UNSUPPORTED naming the limit (lpb_last_error) if not,
+ * LPB_ERR_BAD_ARGUMENT for m <= 0 or n <= 0. */
+int lpb_solve_many_check(int64_t m, int64_t n);
+/* A list of `batch` independent slack-form LPs of different shapes, solved in one call.  m, n: host arrays of
+ * `batch` dims.  A, b, c are packed in list order: LP i's A (row-major, m[i] x n[i]) starts at sum_{k<i} m[k] n[k],
+ * its b at sum_{k<i} m[k], its c at sum_{k<i} n[k]; x_out is packed like c, fun / iterations / status hold `batch`
+ * entries.  `mem` as for lpb_solve_batched.  Each LP gets its own slack structure and the kernel lpb_solve_many
+ * picks for a batch of that LP alone, and its outputs are bit-identical to such a call: the order of the list and
+ * the other LPs in it do not change them.  LPB_ERR_BAD_ARGUMENT for null pointers or non-positive dims,
+ * LPB_ERR_UNSUPPORTED if any LP is outside lpb_solve_many's limits (lpb_last_error names the LP and the limit; the
+ * whole call is refused); both checked before any device is touched. */
+int lpb_solve_many_ragged(int64_t batch, const int64_t* m, const int64_t* n,
+                          const double* A, const double* b, const double* c,
+                          const lpb_options* opts, double* x_out, double* fun,
+                          int64_t* iterations, int32_t* status, int mem, void* stream);
+/* Free the device staging memory lpb_solve_batched / lpb_solve_many / lpb_solve_many_ragged keep between calls with
+ * host inputs, and the page-locked host buffers of lpb_solve_many_ragged (per calling thread). */
 int lpb_release_workspaces(void);
 
 /* ------------------------------------------------------------------ kernel entry points

@@ -119,6 +119,10 @@ SIGNATURES = {
     "lpb_solve_many": (C.c_int, [C.c_int64, C.c_int64, C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p,
                                  C.POINTER(lpb_options), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                  C.c_int, C.c_void_p]),
+    "lpb_solve_many_check": (C.c_int, [C.c_int64, C.c_int64]),
+    "lpb_solve_many_ragged": (C.c_int, [C.c_int64, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                        C.POINTER(lpb_options), C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                        C.c_int, C.c_void_p]),
     "lpb_k_syrk_adat": (C.c_int, [C.c_void_p, C.c_int64, C.c_int64, C.c_void_p, C.c_int64, C.c_void_p,
                                   C.c_void_p, C.c_int64]),
     "lpb_k_potrf": (C.c_int, [C.c_void_p, C.c_int64, C.c_void_p, C.c_int64, c_int32_p]),

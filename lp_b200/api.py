@@ -87,16 +87,20 @@ _BY_CODE = {cls.code: cls for cls in (Unconstrained, NumericalProblem, InvalidPa
                                       IncompatibleInputDimensions, Infeasible, Unbounded)}
 
 
-def _raise_for(code: int, x=None):
-    if code == _ffi.LPB_OK:
-        return
+def _error_for(code: int, x=None) -> Exception:
+    """The exception a non-zero lpb status stands for."""
     if code == _ffi.LPB_ERR_ITERATION_LIMIT_EXCEEDED:
-        raise IterationLimitExceeded(x)
+        return IterationLimitExceeded(x)
     if code in _BY_CODE:
-        raise _BY_CODE[code]()
+        return _BY_CODE[code]()
     if code == _ffi.LPB_ERR_UNSUPPORTED:
-        raise InvalidParameter("unsupported on the B200 path: " + _ffi.last_error())
-    raise DeviceError(code, _ffi.last_error())
+        return InvalidParameter("unsupported on the B200 path: " + _ffi.last_error())
+    return DeviceError(code, _ffi.last_error())
+
+
+def _raise_for(code: int, x=None):
+    if code != _ffi.LPB_OK:
+        raise _error_for(code, x)
 
 
 # --------------------------------------------------------------------------- host buffers
@@ -393,15 +397,100 @@ class InteriorPoint(Solver):
             return OptimizeResult(x.astype(dt), float(dt.type(fun.value)), it.value)
         return OptimizeResult(x, fun.value, it.value)
 
+    def solve_all(self, problems) -> list:
+        """The batched counterpart of `solve`: a list of Problems of any shapes, solved in one call.
+
+        Element i is what `self.solve(problems[i])` returns, except that a LinearProgramError is returned as the
+        exception instance instead of raised.  Problems inside `solve_many`'s limits (m <= 128 and the shared memory
+        their shape needs) go through one `lpb_solve_many_ragged` call: each gets its own slack structure and kernel,
+        and its bits do not depend on the rest of the list.  The others are solved one by one with `solve`.  The
+        problems are packed into a page-locked staging buffer kept per host thread (`release_cached_contexts()`
+        frees it)."""
+        problems = list(problems)
+        out = [None] * len(problems)
+        if not problems:
+            return out
+        lib = _ffi.load()
+        many = [i for i, p in enumerate(problems) if lib.lpb_solve_many_check(*p.A().shape) == _ffi.LPB_OK]
+        if many:
+            pk = _pack_problems([problems[i] for i in many], _staging)
+            batch = len(many)
+            rc = lib.lpb_solve_many_ragged(batch, pk.m.ctypes.data, pk.n.ctypes.data, pk.A.ctypes.data,
+                                           pk.b.ctypes.data, pk.c.ctypes.data, C.byref(self._o), pk.x.ctypes.data,
+                                           pk.fun.ctypes.data, pk.it.ctypes.data, pk.st.ctypes.data,
+                                           _ffi.LPB_MEM_HOST, None)
+            _raise_for(rc)
+            for k, i in enumerate(many):
+                p = problems[i]
+                x_slack = np.array(pk.x[pk.c_off[k]: pk.c_off[k] + pk.n[k]])
+                st = int(pk.st[k])
+                if st != _ffi.LPB_OK:
+                    out[i] = _error_for(st, x_slack)
+                    continue
+                x = x_slack[: len(x_slack) - p.n_slack()]
+                fun = float(pk.fun[k]) + p.c0()  # the kernels leave c0 out: c.x_slack + c0, linear_program.rs:61-63
+                dt = p.dtype()
+                if dt != np.float64:
+                    out[i] = OptimizeResult(x.astype(dt), float(dt.type(fun)), int(pk.it[k]))
+                else:
+                    out[i] = OptimizeResult(x, fun, int(pk.it[k]))
+        for i, p in enumerate(problems):
+            if out[i] is None:
+                try:
+                    out[i] = self.solve(p)
+                except LinearProgramError as e:
+                    out[i] = e
+        return out
+
+
+class _Packed:
+    """A list of slack-form problems packed for lpb_solve_many_ragged: problem k's A (row-major m[k] x n[k]) at
+    a_off[k], b at b_off[k], c and x at c_off[k]; fun / it / st hold one entry per problem."""
+
+
+def _pack_problems(problems, alloc=np.empty) -> _Packed:
+    """Pack `problems` back to back into one float64 buffer from `alloc(count)` (inputs, then outputs)."""
+    pk = _Packed()
+    shapes = np.array([p.A().shape for p in problems], dtype=np.int64).reshape(-1, 2)
+    pk.m, pk.n = np.ascontiguousarray(shapes[:, 0]), np.ascontiguousarray(shapes[:, 1])
+    sizes = pk.m * pk.n
+    pk.a_off = np.concatenate([[0], np.cumsum(sizes)[:-1]]).astype(np.int64)
+    pk.b_off = np.concatenate([[0], np.cumsum(pk.m)[:-1]]).astype(np.int64)
+    pk.c_off = np.concatenate([[0], np.cumsum(pk.n)[:-1]]).astype(np.int64)
+    na, nb, nc, k = int(sizes.sum()), int(pk.m.sum()), int(pk.n.sum()), len(problems)
+    buf = alloc(na + nb + 2 * nc + 3 * k)
+    cuts = np.cumsum([0, na, nb, nc, nc, k, k, k])
+    pk.A, pk.b, pk.c, pk.x = (buf[cuts[i]: cuts[i + 1]] for i in range(4))
+    pk.fun = buf[cuts[4]: cuts[5]]
+    pk.it = buf[cuts[5]: cuts[6]].view(np.int64)
+    pk.st = buf[cuts[6]: cuts[7]].view(np.int32)[:k]
+    for i, p in enumerate(problems):
+        pk.A[pk.a_off[i]: pk.a_off[i] + sizes[i]] = p.A().reshape(-1)
+        pk.b[pk.b_off[i]: pk.b_off[i] + pk.m[i]] = p.b()
+        pk.c[pk.c_off[i]: pk.c_off[i] + pk.n[i]] = p.c()
+    return pk
+
 
 _solve_cache = __import__("threading").local()
 
 
+def _staging(count: int) -> np.ndarray:
+    """`count` float64 of the calling thread's page-locked staging buffer of `solve_all` (grow-only)."""
+    cache = _solve_cache.__dict__
+    buf = cache.get("stage")
+    if buf is None or buf.size < count:
+        cache["stage"] = None
+        buf = cache["stage"] = pinned_empty((count,))
+    return buf[:count]
+
+
 def release_cached_contexts():
-    """Free the device context `InteriorPoint.solve` keeps for the calling thread."""
+    """Free the device context `InteriorPoint.solve` and the staging buffer `InteriorPoint.solve_all` keep for the
+    calling thread."""
     rp = _solve_cache.__dict__.pop("rp", None)
     if rp is not None:
         rp.close()
+    _solve_cache.__dict__.pop("stage", None)
 
 
 class ResidentProblem:

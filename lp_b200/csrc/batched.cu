@@ -12,7 +12,9 @@
 #include "kernels.hpp"
 #include "panel_factor.cuh"
 
+#include <algorithm>
 #include <type_traits>
+#include <vector>
 
 namespace lpb {
 namespace {
@@ -606,21 +608,23 @@ __device__ __forceinline__ void init_dims(Dev& d, int m, int n, int ns) {
   d.ldm = d.mp + 1;
 }
 
-// Loads the rest of problem `lp` (A is in place), runs the driver and writes its outputs.
+// Loads the rest of one LP (A is in place) from gb + b_off and gc + c_off, runs the driver and writes x to
+// x_out + c_off and fun / iterations / status to output slot `slot`.
 template <class Dev>
-__device__ __forceinline__ void solve_one(Dev& d, int64_t lp, const double* __restrict__ gb,
-                                          const double* __restrict__ gc, const lpb_options& opts,
-                                          double* __restrict__ x_out, double* __restrict__ fun_out,
-                                          int64_t* __restrict__ it_out, int32_t* __restrict__ st_out) {
+__device__ __forceinline__ void solve_one(Dev& d, const double* __restrict__ gb, int64_t b_off,
+                                          const double* __restrict__ gc, int64_t c_off, const lpb_options& opts,
+                                          double* __restrict__ x_out, int64_t slot,
+                                          double* __restrict__ fun_out, int64_t* __restrict__ it_out,
+                                          int32_t* __restrict__ st_out) {
   constexpr int kT = Dev::kBT;
   const int m = d.m, n = d.n;
   for (int idx = threadIdx.x; idx < d.mp * d.mp; idx += kT) {  // identity padding of M beyond m (kept by the factorisation)
     const int r = idx / d.mp, cc = idx - r * d.mp;
     if (r >= m || cc >= m) d.M[r * d.ldm + cc] = (r == cc) ? 1.0 : 0.0;
   }
-  for (int i = threadIdx.x; i < m; i += kT) d.b[i] = gb[lp * m + i];
+  for (int i = threadIdx.x; i < m; i += kT) d.b[i] = gb[b_off + i];
   for (int j = threadIdx.x; j < n; j += kT) {
-    d.c[j] = gc[lp * n + j];
+    d.c[j] = gc[c_off + j];
     d.dx[j] = 0.0;
     d.dz[j] = 0.0;
   }
@@ -634,17 +638,47 @@ __device__ __forceinline__ void solve_one(Dev& d, int64_t lp, const double* __re
   if (rc == LPB_OK || rc == LPB_ERR_ITERATION_LIMIT_EXCEEDED) {
     for (int j = threadIdx.x; j < n; j += kT) {
       const double t = d.x[j] / sc.tau;  // mod.rs:231
-      x_out[lp * n + j] = t;
+      x_out[c_off + j] = t;
       f[0] += d.c[j] * t;                // linear_program.rs:62
     }
   }
   block_allreduce<Dev::kBWarps>(f, false, d.red);
   if (threadIdx.x == 0) {
-    fun_out[lp] = f[0];
-    it_out[lp] = sc.iterations;
-    st_out[lp] = rc;
+    fun_out[slot] = f[0];
+    it_out[slot] = sc.iterations;
+    st_out[slot] = rc;
   }
   __syncthreads();
+}
+
+// One LP of m x n with ns implicit slack columns on one CTA (its A at A, the rest located as for solve_one): K6
+// copies the nd = n - ns stored columns of A into shared memory, K8 reads A where it is.  The body of both the uniform
+// and the ragged kernels.
+template <class Dev>
+__device__ __forceinline__ void run_lp(double* sm, int m, int n, int ns, const double* A,
+                                       const double* __restrict__ gb, int64_t b_off, const double* __restrict__ gc,
+                                       int64_t c_off, const lpb_options& opts, double* __restrict__ x_out, int64_t slot,
+                                       double* __restrict__ fun_out, int64_t* __restrict__ it_out,
+                                       int32_t* __restrict__ st_out) {
+  Dev d;
+  init_dims(d, m, n, ns);
+  if constexpr (Dev::kAGlobal) {
+    d.A = A;
+    carve_smem(d, sm);
+  } else {
+    double* sA = sm;
+    d.A = sA;
+    carve_smem(d, sm + (size_t)m * d.lda);
+    for (int idx = threadIdx.x; idx < m * d.nd; idx += Dev::kBT) {
+      const int i = idx / d.nd, j = idx - i * d.nd;
+      sA[i * d.lda + j] = A[i * n + j];
+    }
+    for (int idx = threadIdx.x; idx < m * (d.lda - d.nd); idx += Dev::kBT) {  // zero padding columns: the K tail of the DMMA SYRK
+      const int i = idx / (d.lda - d.nd), j = d.nd + idx - i * (d.lda - d.nd);
+      sA[i * d.lda + j] = 0.0;
+    }
+  }
+  solve_one(d, gb, b_off, gc, c_off, opts, x_out, slot, fun_out, it_out, st_out);
 }
 
 // Two CTAs per SM (128 registers, <= 113 KB of shared memory each) whenever the batch has the slack structure: one LP's
@@ -656,24 +690,8 @@ batched_ipm_kernel(int64_t batch, int m, int n, int ns, const double* __restrict
                    const double* __restrict__ gc, lpb_options opts, double* __restrict__ x_out,
                    double* __restrict__ fun_out, int64_t* __restrict__ it_out, int32_t* __restrict__ st_out) {
   extern __shared__ double sm[];
-  for (int64_t lp = blockIdx.x; lp < batch; lp += gridDim.x) {
-    K6Dev d;
-    init_dims(d, m, n, ns);
-    double* sA = sm;
-    d.A = sA;
-    carve_smem(d, sm + (size_t)m * d.lda);
-
-    const double* A = gA + lp * (int64_t)m * n;
-    for (int idx = threadIdx.x; idx < m * d.nd; idx += kBT) {
-      const int i = idx / d.nd, j = idx - i * d.nd;
-      sA[i * d.lda + j] = A[i * n + j];
-    }
-    for (int idx = threadIdx.x; idx < m * (d.lda - d.nd); idx += kBT) {  // zero padding columns: the K tail of the DMMA SYRK
-      const int i = idx / (d.lda - d.nd), j = d.nd + idx - i * (d.lda - d.nd);
-      sA[i * d.lda + j] = 0.0;
-    }
-    solve_one(d, lp, gb, gc, opts, x_out, fun_out, it_out, st_out);
-  }
+  for (int64_t lp = blockIdx.x; lp < batch; lp += gridDim.x)
+    run_lp<K6Dev>(sm, m, n, ns, gA + lp * (int64_t)m * n, gb, lp * m, gc, lp * n, opts, x_out, lp, fun_out, it_out, st_out);
 }
 
 // K8: LPs of up to 128 rows.  A (m x n, 128 x 256 = 256 KB) no longer fits beside M, so it stays in global memory and
@@ -686,44 +704,92 @@ batched_streamed_kernel(int64_t batch, int m, int n, int ns, const double* __res
                         double* __restrict__ x_out, double* __restrict__ fun_out, int64_t* __restrict__ it_out,
                         int32_t* __restrict__ st_out) {
   extern __shared__ double sm[];
-  for (int64_t lp = blockIdx.x; lp < batch; lp += gridDim.x) {
-    K8Dev d;
-    init_dims(d, m, n, ns);
-    d.A = gA + lp * (int64_t)m * n;
-    carve_smem(d, sm);
-    solve_one(d, lp, gb, gc, opts, x_out, fun_out, it_out, st_out);
-  }
+  for (int64_t lp = blockIdx.x; lp < batch; lp += gridDim.x)
+    run_lp<K8Dev>(sm, m, n, ns, gA + lp * (int64_t)m * n, gb, lp * m, gc, lp * n, opts, x_out, lp, fun_out, it_out, st_out);
 }
 
-// Largest ns such that in EVERY problem of the batch the last ns columns are exactly e_0 .. e_{ns-1} (the slack block
-// ProblemBuilder::build appends, linear_program.rs:145-156).  Detected from the data, never assumed: one CTA per
-// problem finds its own run (columns from the right while column n - ns_lp + r is the unit vector e_r for a
-// consistent ns_lp), the batch takes the minimum.  A batch without the structure gets 0 and the kernel stores all of A.
+// Ragged launch (lpb_solve_many_ragged): a list of LPs of different shapes, one CTA per LP.  CTA k solves LP order[k]:
+// the host decides which LPs start first (the costliest), and the block scheduler hands each freed SM the next LP of
+// the list.  LP lp's dims and offsets come from desc[lp] (x_out uses c's offset); every CTA runs the same arithmetic as
+// the uniform kernel on a batch of that LP alone.
+template <class Dev>
+__device__ __forceinline__ void run_ragged(double* sm, const LpDesc* __restrict__ desc, const int* __restrict__ order,
+                                           const double* __restrict__ gA, const double* __restrict__ gb,
+                                           const double* __restrict__ gc, const lpb_options& opts,
+                                           double* __restrict__ x_out, double* __restrict__ fun_out,
+                                           int64_t* __restrict__ it_out, int32_t* __restrict__ st_out) {
+  const int lp = order[blockIdx.x];
+  const LpDesc e = desc[lp];
+  run_lp<Dev>(sm, e.m, e.n, e.ns, gA + e.a_off, gb, e.b_off, gc, e.c_off, opts, x_out, lp, fun_out, it_out, st_out);
+}
+
+__global__ void __launch_bounds__(kBT, 2)
+ragged_ipm_kernel(const LpDesc* __restrict__ desc, const int* __restrict__ order, const double* __restrict__ gA,
+                  const double* __restrict__ gb, const double* __restrict__ gc, lpb_options opts,
+                  double* __restrict__ x_out, double* __restrict__ fun_out, int64_t* __restrict__ it_out,
+                  int32_t* __restrict__ st_out) {
+  extern __shared__ double sm[];
+  run_ragged<K6Dev>(sm, desc, order, gA, gb, gc, opts, x_out, fun_out, it_out, st_out);
+}
+
+__global__ void __launch_bounds__(kBT8, 1)
+ragged_streamed_kernel(const LpDesc* __restrict__ desc, const int* __restrict__ order, const double* __restrict__ gA,
+                       const double* __restrict__ gb, const double* __restrict__ gc, lpb_options opts,
+                       double* __restrict__ x_out, double* __restrict__ fun_out, int64_t* __restrict__ it_out,
+                       int32_t* __restrict__ st_out) {
+  extern __shared__ double sm[];
+  run_ragged<K8Dev>(sm, desc, order, gA, gb, gc, opts, x_out, fun_out, it_out, st_out);
+}
+
+// Length of the run of trailing columns of one LP (m x n, row-major at A) that are exactly e_0 .. e_{s-1} (the slack
+// block ProblemBuilder::build appends, linear_program.rs:145-156): columns from the right while column n - s + r is
+// the unit vector e_r for a consistent s.  One CTA; the result is in `best` for every thread on return.
+__device__ __forceinline__ void slack_run(const double* __restrict__ A, int m, int n, int smax, int (&urow)[kMaxM8],
+                                          int& best) {  // smax = min(m, n)
+  if (threadIdx.x == 0) best = 0;
+  for (int t = threadIdx.x; t < smax; t += blockDim.x) {  // adjacent threads read adjacent columns of a row: coalesced
+    const int j = n - smax + t;
+    int r = -1;
+    for (int i = 0; i < m; ++i) {
+      const double v = A[(int64_t)i * n + j];
+      if (v != 0.0) r = (v == 1.0 && r == -1) ? i : -2;
+    }
+    urow[t] = r >= 0 ? r : -1;  // urow[t]: column n - smax + t is the unit vector e_{urow[t]} (entry exactly 1), else -1
+  }
+  __syncthreads();
+  for (int s = 1 + threadIdx.x; s <= smax; s += blockDim.x) {  // candidate: the last s columns are e_0 .. e_{s-1}
+    bool good = true;
+    for (int r = 0; r < s; ++r) good = good && urow[smax - s + r] == r;
+    if (good) atomicMax(&best, s);
+  }
+  __syncthreads();
+}
+
+// Largest ns such that in EVERY problem of the batch the last ns columns are exactly e_0 .. e_{ns-1}.  Detected from
+// the data, never assumed: one CTA per problem finds its own run (slack_run), the batch takes the minimum.  A batch
+// without the structure gets 0 and the kernel stores all of A.
 __global__ void __launch_bounds__(256)
 batched_structure_kernel(int64_t batch, int m, int n, const double* __restrict__ gA, int* __restrict__ ns_out) {
-  __shared__ int urow[kMaxM8];  // urow[t]: column n - smax + t is the unit vector e_{urow[t]} (entry exactly 1), else -1
+  __shared__ int urow[kMaxM8];
   __shared__ int best;
   const int smax = m < n ? m : n;
   for (int64_t lp = blockIdx.x; lp < batch; lp += gridDim.x) {
-    const double* A = gA + lp * (int64_t)m * n;
-    if (threadIdx.x == 0) best = 0;
-    for (int t = threadIdx.x; t < smax; t += blockDim.x) {  // adjacent threads read adjacent columns of a row: coalesced
-      const int j = n - smax + t;
-      int r = -1;
-      for (int i = 0; i < m; ++i) {
-        const double v = A[(int64_t)i * n + j];
-        if (v != 0.0) r = (v == 1.0 && r == -1) ? i : -2;
-      }
-      urow[t] = r >= 0 ? r : -1;
-    }
-    __syncthreads();
-    for (int s = 1 + threadIdx.x; s <= smax; s += blockDim.x) {  // candidate: the last s columns are e_0 .. e_{s-1}
-      bool good = true;
-      for (int r = 0; r < s; ++r) good = good && urow[smax - s + r] == r;
-      if (good) atomicMax(&best, s);
-    }
-    __syncthreads();
+    slack_run(gA + lp * (int64_t)m * n, m, n, smax, urow, best);
     if (threadIdx.x == 0) atomicMin(ns_out, best);
+    __syncthreads();
+  }
+}
+
+// The ragged counterpart: every LP of [lo, lo + cnt) keeps its own run, ns_out[lp] (unclamped: the host clamps).
+__global__ void __launch_bounds__(256)
+ragged_structure_kernel(int64_t lo, int64_t cnt, const LpDesc* __restrict__ desc, const double* __restrict__ gA,
+                        int* __restrict__ ns_out) {
+  __shared__ int urow[kMaxM8];
+  __shared__ int best;
+  for (int64_t lp = lo + blockIdx.x; lp < lo + cnt; lp += gridDim.x) {
+    const LpDesc e = desc[lp];
+    slack_run(gA + e.a_off, e.m, e.n, e.m < e.n ? e.m : e.n, urow, best);
+    if (threadIdx.x == 0) ns_out[lp] = best;
     __syncthreads();
   }
 }
@@ -807,6 +873,95 @@ int solve_many_launch(int64_t batch, int m, int n, const double* dA, const doubl
   const int64_t grid = batch < (int64_t)kNumSMs * 64 ? batch : (int64_t)kNumSMs * 64;
   batched_streamed_kernel<<<(unsigned)grid, kBT8, smem, stream>>>(batch, m, n, ns, dA, db, dc, o, dx, dfun, dit, dst);
   LPB_CUDA(cudaGetLastError());
+  return LPB_OK;
+}
+
+// ---------------------------------------------------------------- ragged lists (lpb_solve_many_ragged)
+// Structure scan of LPs [lo, lo + cnt) of a ragged list: ns_dev[lp] = the run of trailing unit columns of LP lp.
+int ragged_scan(int64_t lo, int64_t cnt, const LpDesc* ddesc, const double* dA, int* ns_dev, cudaStream_t stream) {
+  const int64_t sgrid = cnt < (int64_t)kNumSMs * 8 ? cnt : (int64_t)kNumSMs * 8;
+  ragged_structure_kernel<<<(unsigned)sgrid, 256, 0, stream>>>(lo, cnt, ddesc, dA, ns_dev);
+  LPB_CUDA(cudaGetLastError());
+  return LPB_OK;
+}
+
+namespace {
+// Largest dynamic shared memory (bytes) at which ragged_ipm_kernel still runs two CTAs per SM.
+int ragged_two_per_sm_bytes(size_t* out) {
+  int lo = 0, hi = (int)(kSmemCap / sizeof(double));  // in doubles: lo is known to fit twice, hi + 1 not known
+  while (lo < hi) {
+    const int mid = (lo + hi + 1) / 2;
+    int blocks = 0;
+    LPB_CUDA(cudaOccupancyMaxActiveBlocksPerMultiprocessor(&blocks, ragged_ipm_kernel, kBT, (size_t)mid * sizeof(double)));
+    if (blocks >= 2)
+      lo = mid;
+    else
+      hi = mid - 1;
+  }
+  *out = (size_t)lo * sizeof(double);
+  return LPB_OK;
+}
+}  // namespace
+
+// Plans and launches LPs [lo, lo + cnt) of a ragged list, whose raw structure-scan results are in ns_host.  Each LP
+// gets its own clamped ns (written to desc_host) and the kernel solve_many_launch would pick for a batch of that LP
+// alone: K6 where m <= 64 and A fits beside M, else K8.  Up to three launches on `stream`: K8, then the K6 LPs too
+// large for two CTAs per SM, then those that fit two per SM; each with the largest footprint of its group and one CTA
+// per LP, the LPs in descending order of m^2 (n - ns) + m^3 (ties by index), so that the longest solves start first
+// and the short ones fill the tail.  desc_host / order_host [lo, lo + cnt) must be page-locked: they are uploaded to
+// desc_dev / order_dev on `stream`.
+int ragged_launch(int64_t lo, int64_t cnt, LpDesc* desc_host, const int* ns_host, int* order_host, LpDesc* desc_dev,
+                  int* order_dev, const double* dA, const double* db, const double* dc, const lpb_options& o,
+                  double* dx, double* dfun, int64_t* dit, int32_t* dst, cudaStream_t stream) {
+  LPB_CUDA(cudaFuncSetAttribute(ragged_ipm_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemCap));
+  LPB_CUDA(cudaFuncSetAttribute(ragged_streamed_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kSmemCap));
+  size_t two_bytes = 0;
+  LPB_TRY(ragged_two_per_sm_bytes(&two_bytes));
+  enum { kK8 = 0, kK6One = 1, kK6Two = 2 };
+  std::vector<int> grp[3];
+  std::vector<double> cost((size_t)cnt);
+  size_t smem[3] = {0, 0, 0};
+  for (int64_t k = 0; k < cnt; ++k) {
+    LpDesc& e = desc_host[lo + k];
+    int ns = ns_host[lo + k];
+    if (ns < 0 || ns > e.m || ns >= e.n) ns = 0;  // as scan_slack_structure
+    e.ns = ns;
+    int g;
+    size_t bytes;
+    const size_t k6 = batched_smem_doubles(e.m, e.n, ns) * sizeof(double);
+    if (e.m <= kMaxM && k6 <= kSmemCap) {
+      g = k6 <= two_bytes ? kK6Two : kK6One;
+      bytes = k6;
+    } else {
+      g = kK8;
+      bytes = batched_vec_smem_doubles<K8Dev>(e.m, e.n) * sizeof(double);
+    }
+    grp[g].push_back((int)(lo + k));
+    smem[g] = std::max(smem[g], bytes);
+    const double m = e.m;
+    cost[(size_t)k] = m * m * (double)(e.n - ns) + m * m * m;
+  }
+  int* ord = order_host + lo;
+  for (int g = 0; g < 3; ++g) {
+    std::sort(grp[g].begin(), grp[g].end(), [&](int a, int b) {
+      const double ca = cost[(size_t)(a - lo)], cb = cost[(size_t)(b - lo)];
+      return ca > cb || (ca == cb && a < b);
+    });
+    ord = std::copy(grp[g].begin(), grp[g].end(), ord);
+  }
+  LPB_CUDA(cudaMemcpyAsync(desc_dev + lo, desc_host + lo, sizeof(LpDesc) * (size_t)cnt, cudaMemcpyHostToDevice, stream));
+  LPB_CUDA(cudaMemcpyAsync(order_dev + lo, order_host + lo, sizeof(int) * (size_t)cnt, cudaMemcpyHostToDevice, stream));
+  int64_t at = lo;
+  for (int g = 0; g < 3; ++g) {
+    const unsigned grid = (unsigned)grp[g].size();
+    if (grid == 0) continue;
+    if (g == kK8)
+      ragged_streamed_kernel<<<grid, kBT8, smem[g], stream>>>(desc_dev, order_dev + at, dA, db, dc, o, dx, dfun, dit, dst);
+    else
+      ragged_ipm_kernel<<<grid, kBT, smem[g], stream>>>(desc_dev, order_dev + at, dA, db, dc, o, dx, dfun, dit, dst);
+    LPB_CUDA(cudaGetLastError());
+    at += grid;
+  }
   return LPB_OK;
 }
 

@@ -145,4 +145,13 @@ int k_diff(LaunchCtx& lc, const double* a, const double* b, int64_t rows, int64_
 int k_checksum(LaunchCtx& lc, const double* v, int64_t rows, int64_t cols, int64_t ld, int lower_only,
                unsigned long long* out_dev);
 
+// ---------------------------------------------------------------- batched mode, ragged lists (batched.cu)
+// One LP of a list of LPs of different shapes (lpb_solve_many_ragged): its dims, the number ns of trailing columns
+// that are the implicit identity block (0 until the structure scan has run), and where its A (m x n, row-major), b
+// and c start in the packed arrays.  x_out is packed like c.
+struct LpDesc {
+  int m, n, ns, pad;
+  int64_t a_off, b_off, c_off;
+};
+
 }  // namespace lpb

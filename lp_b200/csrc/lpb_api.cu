@@ -28,6 +28,10 @@ int batched_launch(int64_t batch, int m, int n, const double* dA, const double* 
 int solve_many_check_shape(int64_t m, int64_t n);
 int solve_many_launch(int64_t batch, int m, int n, const double* dA, const double* db, const double* dc,
                       const lpb_options& o, double* dx, double* dfun, int64_t* dit, int32_t* dst, cudaStream_t stream);
+int ragged_scan(int64_t lo, int64_t cnt, const LpDesc* ddesc, const double* dA, int* ns_dev, cudaStream_t stream);
+int ragged_launch(int64_t lo, int64_t cnt, LpDesc* desc_host, const int* ns_host, int* order_host, LpDesc* desc_dev,
+                  int* order_dev, const double* dA, const double* db, const double* dc, const lpb_options& o,
+                  double* dx, double* dfun, int64_t* dit, int32_t* dst, cudaStream_t stream);
 }
 
 using namespace lpb;
@@ -170,11 +174,15 @@ struct ProcessComm {
 ProcessComm g_comm;
 std::mutex g_comm_mu;
 
-// device staging arena of lpb_solve_batched / lpb_solve_many for host inputs (per host thread, grow-only)
+// device staging arena of lpb_solve_batched / lpb_solve_many / lpb_solve_many_ragged for host inputs (per host
+// thread, grow-only); the ragged call also keeps its descriptors, structure results and launch order there
 thread_local void* g_batched_ws = nullptr;
 thread_local cudaStream_t g_batched_copy_stream = nullptr;  // uploads of host inputs, see run_batched
 thread_local cudaEvent_t g_batched_ev[4] = {nullptr, nullptr, nullptr, nullptr};
 thread_local size_t g_batched_ws_cap = 0;
+// page-locked host side of the ragged call's descriptors, structure results and launch order (grow-only)
+thread_local void* g_ragged_host = nullptr;
+thread_local size_t g_ragged_host_cap = 0;
 
 int allreduce(lpb_ctx* c, double* buf, int64_t count, ncclRedOp_t op) {
   if (c->world <= 1) return LPB_OK;
@@ -778,6 +786,39 @@ int need_problem(lpb_ctx* c) {
   return LPB_OK;
 }
 
+size_t carve_up(size_t v) { return (v + 255) & ~(size_t)255; }
+
+// Consecutive 256-byte aligned pieces of the staging arena.
+struct Carver {
+  char* p = nullptr;
+  char* operator()(size_t bytes) {
+    char* r = p;
+    p += carve_up(bytes);
+    return r;
+  }
+};
+
+// The per-thread staging arena, grown to at least `need` bytes (its contents are not kept).
+int batched_arena(size_t need, Carver* out) {
+  if (g_batched_ws_cap < need) {
+    if (g_batched_ws) cudaFree(g_batched_ws);
+    g_batched_ws = nullptr;
+    g_batched_ws_cap = 0;
+    LPB_CUDA(cudaMalloc(&g_batched_ws, need));
+    g_batched_ws_cap = need;
+  }
+  out->p = static_cast<char*>(g_batched_ws);
+  return LPB_OK;
+}
+
+// The per-thread copy stream of host-input uploads and the four chunk events
+int batched_copy_stream() {
+  if (!g_batched_copy_stream) LPB_CUDA(cudaStreamCreateWithFlags(&g_batched_copy_stream, cudaStreamNonBlocking));
+  for (int q = 0; q < 4; ++q)
+    if (!g_batched_ev[q]) LPB_CUDA(cudaEventCreateWithFlags(&g_batched_ev[q], cudaEventDisableTiming));
+  return LPB_OK;
+}
+
 using BatchedLaunch = int (*)(int64_t, int, int, const double*, const double*, const double*, const lpb_options&, double*,
                               double*, int64_t*, int32_t*, cudaStream_t);
 
@@ -796,21 +837,8 @@ int run_batched(BatchedLaunch launch, int64_t batch, int64_t m, int64_t n, const
   const size_t sA = sizeof(double) * (size_t)(batch * m * n), sb = sizeof(double) * (size_t)(batch * m),
                sc = sizeof(double) * (size_t)(batch * n), s8 = sizeof(double) * (size_t)batch,
                s4 = sizeof(int32_t) * (size_t)batch;
-  auto up = [](size_t v) { return (v + 255) & ~(size_t)255; };
-  const size_t need = up(sA) + up(sb) + 2 * up(sc) + 2 * up(s8) + up(s4);
-  if (g_batched_ws_cap < need) {
-    if (g_batched_ws) cudaFree(g_batched_ws);
-    g_batched_ws = nullptr;
-    g_batched_ws_cap = 0;
-    LPB_CUDA(cudaMalloc(&g_batched_ws, need));
-    g_batched_ws_cap = need;
-  }
-  char* p = static_cast<char*>(g_batched_ws);
-  auto carve = [&](size_t bytes) {
-    char* r = p;
-    p += up(bytes);
-    return r;
-  };
+  Carver carve;
+  LPB_TRY(batched_arena(carve_up(sA) + carve_up(sb) + 2 * carve_up(sc) + 2 * carve_up(s8) + carve_up(s4), &carve));
   double* dA = reinterpret_cast<double*>(carve(sA));
   double* db = reinterpret_cast<double*>(carve(sb));
   double* dc = reinterpret_cast<double*>(carve(sc));
@@ -822,9 +850,7 @@ int run_batched(BatchedLaunch launch, int64_t batch, int64_t m, int64_t n, const
   // own upload only, so the upload of chunk i + 1 (PCIe) runs under the kernel of chunk i and the downloads of chunk
   // i - 1.  At C4 the upload (558 MB, ~10 ms from pinned memory) and the kernel (~11 ms) used to add up.
   const int64_t nchunk = batch >= 1024 ? 4 : 1;
-  if (!g_batched_copy_stream) LPB_CUDA(cudaStreamCreateWithFlags(&g_batched_copy_stream, cudaStreamNonBlocking));
-  for (int q = 0; q < 4; ++q)
-    if (!g_batched_ev[q]) LPB_CUDA(cudaEventCreateWithFlags(&g_batched_ev[q], cudaEventDisableTiming));
+  LPB_TRY(batched_copy_stream());
   LPB_CUDA(cudaEventRecord(g_batched_ev[0], st));  // the copy stream starts behind whatever `st` holds already
   LPB_CUDA(cudaStreamWaitEvent(g_batched_copy_stream, g_batched_ev[0], 0));
   auto lo = [&](int64_t q) { return batch * q / nchunk; };
@@ -864,6 +890,92 @@ int batched_args(const char* who, int64_t batch, int64_t m, int64_t n, const dou
   else
     options_default(o);
   return lpb_options_validate(o);
+}
+
+// A ragged list (lpb_solve_many_ragged) on device arrays, or with host arrays staged through the per-thread arena as
+// in run_batched.  Per chunk: its upload, then its structure scan and the download of the scan's results, on the copy
+// stream; the host waits for those results (while the previous chunk's kernels run), plans the chunk and queues its
+// launches and downloads on `st`.  Device inputs are one chunk, scanned on `st`: one synchronisation before the plan.
+int run_ragged(int64_t batch, const int64_t* m, const int64_t* n, const double* A, const double* b, const double* c,
+               const lpb_options& o, double* x_out, double* fun, int64_t* iterations, int32_t* status, int mem,
+               cudaStream_t st) {
+  const bool host = mem != LPB_MEM_DEVICE;
+  const size_t sd = sizeof(LpDesc) * (size_t)batch, si = sizeof(int) * (size_t)batch;
+  if (g_ragged_host_cap < sd + 2 * si) {
+    if (g_ragged_host) cudaFreeHost(g_ragged_host);
+    g_ragged_host = nullptr;
+    g_ragged_host_cap = 0;
+    LPB_CUDA(cudaMallocHost(&g_ragged_host, sd + 2 * si));
+    g_ragged_host_cap = sd + 2 * si;
+  }
+  LpDesc* hdesc = static_cast<LpDesc*>(g_ragged_host);
+  int* hns = reinterpret_cast<int*>(hdesc + batch);
+  int* hord = hns + batch;
+  int64_t nA = 0, nb = 0, nc = 0;  // packed lengths
+  for (int64_t i = 0; i < batch; ++i) {
+    hdesc[i] = LpDesc{(int)m[i], (int)n[i], 0, 0, nA, nb, nc};
+    nA += m[i] * n[i];
+    nb += m[i];
+    nc += n[i];
+  }
+  const size_t sA = sizeof(double) * (size_t)nA, sb = sizeof(double) * (size_t)nb, sc = sizeof(double) * (size_t)nc,
+               s8 = sizeof(double) * (size_t)batch, s4 = sizeof(int32_t) * (size_t)batch;
+  size_t need = carve_up(sd) + 2 * carve_up(si);
+  if (host) need += carve_up(sA) + carve_up(sb) + 2 * carve_up(sc) + 2 * carve_up(s8) + carve_up(s4);
+  Carver carve;
+  LPB_TRY(batched_arena(need, &carve));
+  LpDesc* ddesc = reinterpret_cast<LpDesc*>(carve(sd));
+  int* dns = reinterpret_cast<int*>(carve(si));
+  int* dord = reinterpret_cast<int*>(carve(si));
+  const double* dA = host ? reinterpret_cast<double*>(carve(sA)) : A;
+  const double* db = host ? reinterpret_cast<double*>(carve(sb)) : b;
+  const double* dc = host ? reinterpret_cast<double*>(carve(sc)) : c;
+  double* dx = host ? reinterpret_cast<double*>(carve(sc)) : x_out;
+  double* df = host ? reinterpret_cast<double*>(carve(s8)) : fun;
+  int64_t* dit = host ? reinterpret_cast<int64_t*>(carve(s8)) : iterations;
+  int32_t* dst = host ? reinterpret_cast<int32_t*>(carve(s4)) : status;
+  LPB_TRY(batched_copy_stream());
+  cudaStream_t cs = st;
+  if (host) {
+    cs = g_batched_copy_stream;
+    LPB_CUDA(cudaEventRecord(g_batched_ev[0], st));  // the copy stream starts behind whatever `st` holds already
+    LPB_CUDA(cudaStreamWaitEvent(cs, g_batched_ev[0], 0));
+  }
+  // chunks by LP count; [a_off, b_off, c_off) of LP `lo(q)` .. the end of the packed arrays for q = nchunk
+  const int64_t nchunk = host && batch >= 1024 ? 4 : 1;
+  auto lo = [&](int64_t q) { return batch * q / nchunk; };
+  auto off = [&](int64_t i, int which) -> int64_t {
+    if (i == batch) return which == 0 ? nA : which == 1 ? nb : nc;
+    return which == 0 ? hdesc[i].a_off : which == 1 ? hdesc[i].b_off : hdesc[i].c_off;
+  };
+  LPB_CUDA(cudaMemcpyAsync(ddesc, hdesc, sd, cudaMemcpyHostToDevice, cs));
+  for (int64_t q = 0; q < nchunk; ++q) {
+    const int64_t l0 = lo(q), l1 = lo(q + 1);
+    if (host) {
+      const double* src[3] = {A, b, c};
+      const double* dst3[3] = {dA, db, dc};
+      for (int w = 0; w < 3; ++w)
+        LPB_CUDA(cudaMemcpyAsync(const_cast<double*>(dst3[w]) + off(l0, w), src[w] + off(l0, w),
+                                 sizeof(double) * (size_t)(off(l1, w) - off(l0, w)), cudaMemcpyHostToDevice, cs));
+    }
+    LPB_TRY(ragged_scan(l0, l1 - l0, ddesc, dA, dns, cs));
+    LPB_CUDA(cudaMemcpyAsync(hns + l0, dns + l0, sizeof(int) * (size_t)(l1 - l0), cudaMemcpyDeviceToHost, cs));
+    LPB_CUDA(cudaEventRecord(g_batched_ev[q], cs));
+  }
+  for (int64_t q = 0; q < nchunk; ++q) {
+    const int64_t l0 = lo(q), l1 = lo(q + 1);
+    LPB_CUDA(cudaEventSynchronize(g_batched_ev[q]));
+    if (host) LPB_CUDA(cudaStreamWaitEvent(st, g_batched_ev[q], 0));
+    LPB_TRY(ragged_launch(l0, l1 - l0, hdesc, hns, hord, ddesc, dord, dA, db, dc, o, dx, df, dit, dst, st));
+    if (!host) continue;
+    const int64_t x0 = off(l0, 2), x1 = off(l1, 2);
+    LPB_CUDA(cudaMemcpyAsync(x_out + x0, dx + x0, sizeof(double) * (size_t)(x1 - x0), cudaMemcpyDeviceToHost, st));
+    LPB_CUDA(cudaMemcpyAsync(fun + l0, df + l0, sizeof(double) * (size_t)(l1 - l0), cudaMemcpyDeviceToHost, st));
+    LPB_CUDA(cudaMemcpyAsync(iterations + l0, dit + l0, sizeof(int64_t) * (size_t)(l1 - l0), cudaMemcpyDeviceToHost, st));
+    LPB_CUDA(cudaMemcpyAsync(status + l0, dst + l0, sizeof(int32_t) * (size_t)(l1 - l0), cudaMemcpyDeviceToHost, st));
+  }
+  LPB_CUDA(cudaStreamSynchronize(st));
+  return LPB_OK;
 }
 }  // namespace
 
@@ -1400,10 +1512,55 @@ int lpb_solve_many(int64_t batch, int64_t m, int64_t n, const double* A, const d
                      static_cast<cudaStream_t>(stream));
 }
 
+int lpb_solve_many_check(int64_t m, int64_t n) {
+  if (m <= 0 || n <= 0) {
+    set_last_error("solve_many: non-positive size (m = %lld, n = %lld)", (long long)m, (long long)n);
+    return LPB_ERR_BAD_ARGUMENT;
+  }
+  return solve_many_check_shape(m, n);
+}
+
+int lpb_solve_many_ragged(int64_t batch, const int64_t* m, const int64_t* n, const double* A, const double* b,
+                          const double* c, const lpb_options* opts, double* x_out, double* fun, int64_t* iterations,
+                          int32_t* status, int mem, void* stream) {
+  if (batch <= 0 || !m || !n || !A || !b || !c || !x_out || !fun || !iterations || !status) {
+    set_last_error("solve_many_ragged: null pointer or non-positive size");
+    return LPB_ERR_BAD_ARGUMENT;
+  }
+  if (batch > INT32_MAX) {  // one CTA per LP, indexed by int
+    set_last_error("solve_many_ragged: at most %d LPs per call (got %lld)", INT32_MAX, (long long)batch);
+    return LPB_ERR_UNSUPPORTED;
+  }
+  for (int64_t i = 0; i < batch; ++i) {
+    if (m[i] <= 0 || n[i] <= 0) {
+      set_last_error("solve_many_ragged: LP %lld has m = %lld, n = %lld", (long long)i, (long long)m[i], (long long)n[i]);
+      return LPB_ERR_BAD_ARGUMENT;
+    }
+  }
+  for (int64_t i = 0; i < batch; ++i) {  // shape limits first: they hold or fail without a device
+    if (solve_many_check_shape(m[i], n[i]) != LPB_OK) {
+      const std::string why = get_last_error();
+      set_last_error("solve_many_ragged: LP %lld: %s", (long long)i, why.c_str());
+      return LPB_ERR_UNSUPPORTED;
+    }
+  }
+  lpb_options o;
+  if (opts)
+    o = *opts;
+  else
+    options_default(&o);
+  LPB_TRY(lpb_options_validate(&o));
+  LPB_TRY(check_device());
+  return run_ragged(batch, m, n, A, b, c, o, x_out, fun, iterations, status, mem, static_cast<cudaStream_t>(stream));
+}
+
 int lpb_release_workspaces(void) {
   if (g_batched_ws) cudaFree(g_batched_ws);
   g_batched_ws = nullptr;
   g_batched_ws_cap = 0;
+  if (g_ragged_host) cudaFreeHost(g_ragged_host);
+  g_ragged_host = nullptr;
+  g_ragged_host_cap = 0;
   if (g_batched_copy_stream) cudaStreamDestroy(g_batched_copy_stream);
   g_batched_copy_stream = nullptr;
   for (int q = 0; q < 4; ++q) {
